@@ -6,6 +6,7 @@ obj_proj -> similarity scoring).  Default workload = BASELINE.json configs[2] (1
   python bench.py --config c1|c2|c3|c4 ...                           # the other BASELINE.json configurations
   torchrun ... bench.py --gpus N ...                                 # one rank per GPU, weak scaling, 1 all-gather / step
   python bench.py --impl reference ...                               # reference algorithm on the host CPU cores
+  python bench.py ... --dump-outputs DIR                             # also write the last timed step's outputs, DIR/*.npy
 
 One JSON line is printed by rank 0 (contract: task description / DESIGN.md section "Measurement").
 
@@ -142,6 +143,26 @@ def gpu_ms(fn, iters=5, warm=2):
     return e0.elapsed_time(e1) / iters
 
 
+def write_outputs(out_dir, arrays, sample=1 << 20, limit=64 << 20):
+    """--dump-outputs: each tensor of `arrays` (name -> tensor) as <out_dir>/<name>.npy, floating point as float32 and
+    integers as float64 (exact).  A tensor of more than `sample` elements is written as its flattened values at `sample`
+    positions drawn from a fixed seed: the same positions in every run, so that two builds compare element for element."""
+    import numpy as np
+    host = {}
+    for name, t in arrays.items():
+        t = t.detach()
+        t = t.double() if t.dtype == torch.float64 or not t.is_floating_point() else t.float()
+        if t.numel() > sample:
+            idx = torch.randint(t.numel(), (sample,), generator=torch.Generator().manual_seed(0)).sort().values
+            t = t.flatten()[idx.to(t.device)]
+        host[name] = t.cpu().numpy()
+    total = sum(a.nbytes for a in host.values())
+    assert total <= limit, "--dump-outputs: %d bytes of outputs, more than %d" % (total, limit)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in host.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 # ---------------------------------------------------------------------------------------------- model construction
 def build_modules(frames, nq, seed=0, pred_traj=False, device=None):
     """Random-init L/14 video tower + object decoder.  device=None: parameters drawn on the host from a seeded generator
@@ -203,7 +224,7 @@ def run_reference(args, cfg, rank, emit):
     sample = 4                                    # ~10 s of host work per step on a 16-core box at 16 frames
     for _ in range(min(args.warmup, 1)):
         cpu_forward_clips(vsd, dsd, T, sample, cores, nq, cfg["pred_traj"])
-    steps = max(1, min(args.steps, 3))
+    steps = args.steps
     dts = [cpu_forward_clips(vsd, dsd, T, sample, cores, nq, cfg["pred_traj"]) for _ in range(steps)]
     dt = sum(dts) / len(dts)
     val = sample / dt
@@ -321,6 +342,8 @@ class TrainShare:
             lo_, _ = box_utils.compute_box_loss('obj_boxes', self.crit, mo, self.px[:, 2:].clone(), None, self.sizes, n_queries=12)
             word = loss.WordContrastiveLoss()(self.model.txt_proj(self.noun_feats), emb[:, :-1].contiguous(), self.inds)
         total = nce + lh + lo_ + 0.5 * word
+        self.outputs = {"loss": total, "video_embed": vid, "text_embed": txt, "pred_boxes": mo["pred_boxes"],
+                        "pred_logits": mo["pred_logits"]}
         if ev:
             ev[3].record()
         with around("backward"):
@@ -474,13 +497,23 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip gpu_eager_baseline and the extra.* measurements")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed as DIR/<name>.npy (rank 0; outputs "
+                         "of more than 2^20 elements as a fixed, seeded sample of their elements)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the GPU path (--impl b200)")
     cfg = dict(CONFIGS[args.config])
     for k in ("batch", "frames", "nq"):
         if getattr(args, k) is not None:
             cfg[k] = getattr(args, k)
 
     rank, world, local = env_int("RANK", 0), env_int("WORLD_SIZE", 1), env_int("LOCAL_RANK", 0)
+    # inputs the configurations draw from torch's default generators (c3's embedding bank) and the decoder's dropout
+    # stream in train() mode (c4) follow this seed: the same arguments give the same computation in every run
+    torch.manual_seed(rank)
     # stdout carries exactly one JSON line: while the benchmark runs, file descriptor 1 points at stderr, so that
     # anything a C library prints there (NCCL's "NCCL version ..." banner when the box sets NCCL_DEBUG) cannot end up in
     # front of it; the descriptor is restored for the final print
@@ -662,6 +695,12 @@ def run_forward(ctx):
     dec.set_profile(False)
     ms_step = ms_total / args.steps
     value = world * B / (ms_step * 1e-3)
+    if args.dump_outputs and rank == 0:
+        # the e2e measurements below take more steps: the timed path's last outputs are written now.  The step keeps
+        # only its embeddings and choices; the scores it ranked are recomputed from them by the same kernel
+        allv, res = state["last"]
+        sim = metric.sim_matrix(text_bank if mir_rows else text, allv)
+        write_outputs(args.dump_outputs, {"video_embed": allv, "sim": sim, "choice": res})
 
     # ---- end to end through the public modules with host buffers: pinned H2D of the clips + D2H of the choices
     e2e = e2e_u8 = None
@@ -841,6 +880,9 @@ def run_train(ctx):
         sampler.start()
     ms_total, _, per_rank = timed(lambda: ts.step(), args.steps)
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        params = torch.cat([p.detach().flatten() for p in ts.model.parameters()])    # after the last optimizer step
+        write_outputs(args.dump_outputs, dict(ts.outputs, decoder_params=params))
     ms_step = ms_total / args.steps
     value = world * B / (ms_step * 1e-3)
     ts.step(timed_parts=True)

@@ -1,6 +1,6 @@
-"""Generate tests/golden/*.pt by running the UNMODIFIED reference (build container only).
+"""Generate tests/golden/*.pt by running the UNMODIFIED reference (a checkout of the original project).
 
-TEST INFRASTRUCTURE ONLY.  Usage:  python -m oracle.make_golden  [--check]
+TEST INFRASTRUCTURE ONLY.  Usage:  HH_REFERENCE_ROOT=<checkout> python -m oracle.make_golden  [--check]
 
 Each fixture holds the *reference's* outputs for a seeded synthetic state_dict + input (both
 regenerated from the seed by `hh_oracle.synth_state_dict` / `golden_cases.make_inputs`, so only the

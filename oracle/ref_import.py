@@ -1,8 +1,8 @@
-"""Import the *unmodified* reference modules from /root/reference (build container only).
+"""Import the *unmodified* reference modules from a checkout of the original project named by $HH_REFERENCE_ROOT.
 
-TEST INFRASTRUCTURE ONLY.  /root/reference does not exist on the GPU box, so nothing
+TEST INFRASTRUCTURE ONLY.  The original project is not part of this repository, so nothing
 reachable from `pytest -m gpu`, smoke() or bench.py may call into this file; it is used
-by `oracle/make_golden.py` and by the CPU tests that are skipped when the tree is absent.
+by `oracle/make_golden.py` and by the CPU tests that are skipped when no checkout is named.
 
 The reference imports two packages the image lacks (SURVEY.md §8c):
   * ``timm.models.layers`` -- only DropPath / to_2tuple / trunc_normal_ are used
@@ -18,11 +18,11 @@ import types
 import contextlib
 import io
 
-REFERENCE_ROOT = os.environ.get("HH_REFERENCE_ROOT", "/root/reference")
+REFERENCE_ROOT = os.environ.get("HH_REFERENCE_ROOT", "")
 
 
 def reference_available() -> bool:
-    return os.path.isfile(os.path.join(REFERENCE_ROOT, "model", "LaviLa.py"))
+    return bool(REFERENCE_ROOT) and os.path.isfile(os.path.join(REFERENCE_ROOT, "model", "LaviLa.py"))
 
 
 def _install_shims():
@@ -67,7 +67,7 @@ def _install_shims():
 def import_reference():
     """Returns a namespace with the reference modules (LaviLa, tfm_decoder, metric, box_ops, ...)."""
     if not reference_available():
-        raise RuntimeError("reference tree not present at %s" % REFERENCE_ROOT)
+        raise RuntimeError("HH_REFERENCE_ROOT (%r) does not name a checkout of the original project" % REFERENCE_ROOT)
     _install_shims()
     if REFERENCE_ROOT not in sys.path:
         sys.path.insert(0, REFERENCE_ROOT)

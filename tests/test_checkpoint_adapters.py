@@ -1,5 +1,10 @@
-"""Host-side checkpoint adapters (SURVEY.md section 8f row 4) against the reference's own functions."""
+"""Host-side checkpoint adapters (SURVEY.md section 8f row 4) against the reference's own functions.
+
+tests/golden/checkpoint_adapters.pt holds what the comparison with the reference looks at (_adapter_outputs): it was
+recorded from this repository's adapters, is compared with them everywhere, and is itself compared with the original
+project's functions by the live test whenever $HH_REFERENCE_ROOT names a checkout of it."""
 import ast
+import os
 
 import pytest
 import torch
@@ -23,6 +28,33 @@ def _clip_visual_sd(layers=2, width=8):
                        ("mlp.c_proj.weight", (width, 4 * width)), ("mlp.c_proj.bias", (width,))):
             sd[p + k] = torch.randn(*shp, generator=g)
     return sd
+
+
+GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "checkpoint_adapters.pt")
+INFLATE_CASES = [(4, 16, "bilinear"), (4, 16, "interp"), (4, 16, "zeros"), (16, 4, "bilinear"), (4, 4, "zeros")]
+
+
+def _adapter_outputs(remap_keys, inflate_positional_embeds):
+    out = {"remap_keys": remap_keys(_clip_visual_sd(), transformer_layers=2)}
+    for have, want_t, fix in INFLATE_CASES:
+        cur = {"visual.temporal_embed": torch.zeros(1, want_t, 8)}
+        new = {"visual.temporal_embed": torch.arange(have * 8.).view(1, have, 8)}
+        out["inflate_%d_%d_%s" % (have, want_t, fix)] = inflate_positional_embeds(
+            cur, new, num_frames=want_t, load_temporal_fix=fix)["visual.temporal_embed"]
+    return out
+
+
+def _assert_same(got, want):
+    assert list(got) == list(want)
+    assert list(got["remap_keys"]) == list(want["remap_keys"])
+    assert all(torch.equal(got["remap_keys"][k], v) for k, v in want["remap_keys"].items())
+    for k, v in want.items():
+        if k != "remap_keys":
+            assert torch.equal(got[k], v), k
+
+
+def test_adapters_equal_the_stored_reference_outputs():
+    _assert_same(_adapter_outputs(ck.remap_keys, ck.inflate_positional_embeds), torch.load(GOLDEN))
 
 
 def test_strip_module_prefix():
@@ -51,21 +83,14 @@ def test_inflate_contract():
         ck.inflate_positional_embeds(cur, {"visual.temporal_embed": torch.zeros(1, 4, 8)}, num_frames=8)
 
 
-@pytest.mark.skipif(not ref_import.reference_available(), reason="reference tree only exists in the build container")
+@pytest.mark.skipif(not ref_import.reference_available(), reason="needs a checkout of the original project (HH_REFERENCE_ROOT)")
 def test_adapters_equal_the_reference(capsys):
     ns = ref_import.import_reference()
-    want = ns.LaviLa.remap_keys(_clip_visual_sd(), transformer_layers=2)
-    got = ck.remap_keys(_clip_visual_sd(), transformer_layers=2)
-    assert list(got) == list(want) and all(torch.equal(got[k], want[k]) for k in want)
     # run/test_egtea.py imports sacred at module level; execute only its inflate_positional_embeds definition
     src = open(ref_import.REFERENCE_ROOT + "/run/test_egtea.py").read()
     fn = next(n for n in ast.parse(src).body if isinstance(n, ast.FunctionDef) and n.name == "inflate_positional_embeds")
     scope = {"torch": torch, "F": torch.nn.functional}
     exec(compile(ast.Module(body=[fn], type_ignores=[]), "ref_inflate", "exec"), scope)
-    for have, want_t, fix in [(4, 16, "bilinear"), (4, 16, "interp"), (4, 16, "zeros"), (16, 4, "bilinear"), (4, 4, "zeros")]:
-        cur = {"visual.temporal_embed": torch.zeros(1, want_t, 8)}
-        a = scope["inflate_positional_embeds"](cur, {"visual.temporal_embed": torch.arange(have * 8.).view(1, have, 8)},
-                                               num_frames=want_t, load_temporal_fix=fix)
-        b = ck.inflate_positional_embeds(cur, {"visual.temporal_embed": torch.arange(have * 8.).view(1, have, 8)},
-                                         num_frames=want_t, load_temporal_fix=fix)
-        assert torch.equal(a["visual.temporal_embed"], b["visual.temporal_embed"]), (have, want_t, fix)
+    want = _adapter_outputs(ns.LaviLa.remap_keys, scope["inflate_positional_embeds"])
+    _assert_same(_adapter_outputs(ck.remap_keys, ck.inflate_positional_embeds), want)
+    _assert_same(torch.load(GOLDEN), want)

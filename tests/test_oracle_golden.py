@@ -2,7 +2,7 @@
 
 * everywhere: against the committed fixtures in tests/golden/ (made by oracle/make_golden.py from the
   unmodified reference);
-* in the build container (where /root/reference exists): against the live reference as well.
+* where $HH_REFERENCE_ROOT names a checkout of the original project: against the live reference as well.
 """
 import os
 
@@ -35,7 +35,7 @@ def test_oracle_matches_golden_fixture(name):
     _compare(ref, gc.run_oracle(gc.CASES[name]), name)
 
 
-@pytest.mark.skipif(not ref_import.reference_available(), reason="reference tree only exists in the build container")
+@pytest.mark.skipif(not ref_import.reference_available(), reason="needs a checkout of the original project (HH_REFERENCE_ROOT)")
 @pytest.mark.parametrize("name", ["enc_tiny", "enc_l14", "enc_l14_t16", "dec_tiny_traj", "dec_tiny_notraj", "dec_train_dropout", "boxes", "score", "losses"])
 def test_fixture_is_what_the_live_reference_says(name):
     from oracle import make_golden
