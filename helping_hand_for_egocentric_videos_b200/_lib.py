@@ -41,6 +41,8 @@ SIGNATURES = {
     "hh_encoder_forward": (_i, [_p, _p, _i, _p, _p]),
     "hh_encoder_forward_n": (_i, [_p, _p, _i, _i, _p, _p]),
     "hh_encoder_forward_u8": (_i, [_p, _p, _i, C.POINTER(_f), C.POINTER(_f), _p, _p]),
+    "hh_encoder_forward_bf16": (_i, [_p, _p, _i, _p, _p, _p]),
+    "hh_encoder_forward_u8_bf16": (_i, [_p, _p, _i, C.POINTER(_f), C.POINTER(_f), _p, _p, _p]),
     "hh_encoder_flops_per_clip": (C.c_double, [_p]),
     "hh_encoder_last_launches": (_i, [_p]),
     "hh_decoder_create": (_i, [C.POINTER(_p), C.POINTER(DecoderCfg)]),
@@ -48,6 +50,8 @@ SIGNATURES = {
     "hh_decoder_set_weight": (_i, [_p, C.c_char_p, _p, _i64, _p]),
     "hh_decoder_forward": (_i, [_p, _p, _i64, _i64, _i, _i, _p, _p, _p, _p]),
     "hh_decoder_forward_train": (_i, [_p, _p, _i64, _i64, _i, _i, _p, _p, _p, _p]),
+    "hh_decoder_forward_bf16": (_i, [_p, _p, _i64, _i64, _i, _i, _p, _p, _p, _p]),
+    "hh_decoder_forward_train_bf16": (_i, [_p, _p, _i64, _i64, _i, _i, _p, _p, _p, _p]),
     "hh_decoder_set_dropout": (_i, [_p, _f, C.c_uint64, C.c_uint32]),
     "hh_decoder_backward": (_i, [_p, _p, _p, _p, _p, _p]),
     "hh_decoder_generation": (C.c_uint64, [_p]),

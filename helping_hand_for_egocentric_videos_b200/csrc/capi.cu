@@ -58,7 +58,9 @@ int hh_encoder_set_weight(hh_encoder* enc, const char* key, const float* data, i
 int hh_encoder_forward_n(hh_encoder* enc, const float* video, int B, int nblocks, float* fmap, void* stream) {
   HH_GUARD_BEGIN
   if (!enc) return fail(-1, "hh_encoder_forward: null handle");
-  return enc->impl.forward(video, B, nblocks, fmap, S(stream));
+  Encoder::Fmap o;
+  o.f32 = fmap;
+  return enc->impl.forward(video, B, nblocks, o, S(stream));
   HH_GUARD_END
 }
 int hh_encoder_forward(hh_encoder* enc, const float* video, int B, float* fmap, void* stream) {
@@ -68,7 +70,28 @@ int hh_encoder_forward_u8(hh_encoder* enc, const uint8_t* frames, int B, const f
                           void* stream) {
   HH_GUARD_BEGIN
   if (!enc) return fail(-1, "hh_encoder_forward_u8: null handle");
-  return enc->impl.forward_u8(frames, mean, stdv, B, fmap, S(stream));
+  Encoder::Fmap o;
+  o.f32 = fmap;
+  return enc->impl.forward_u8(frames, mean, stdv, B, o, S(stream));
+  HH_GUARD_END
+}
+int hh_encoder_forward_bf16(hh_encoder* enc, const float* video, int B, void* fmap, float* cls, void* stream) {
+  HH_GUARD_BEGIN
+  if (!enc) return fail(-1, "hh_encoder_forward_bf16: null handle");
+  Encoder::Fmap o;
+  o.b16 = static_cast<bf16*>(fmap);
+  o.cls = cls;
+  return enc->impl.forward(video, B, -1, o, S(stream));
+  HH_GUARD_END
+}
+int hh_encoder_forward_u8_bf16(hh_encoder* enc, const uint8_t* frames, int B, const float* mean, const float* stdv,
+                               void* fmap, float* cls, void* stream) {
+  HH_GUARD_BEGIN
+  if (!enc) return fail(-1, "hh_encoder_forward_u8_bf16: null handle");
+  Encoder::Fmap o;
+  o.b16 = static_cast<bf16*>(fmap);
+  o.cls = cls;
+  return enc->impl.forward_u8(frames, mean, stdv, B, o, S(stream));
   HH_GUARD_END
 }
 double hh_encoder_flops_per_clip(const hh_encoder* enc) { return enc ? enc->impl.flops_per_clip() : 0.0; }
@@ -96,14 +119,28 @@ int hh_decoder_forward(hh_decoder* dec, const float* features, int64_t stride_b,
                        float* hs, float* logits, float* boxes, void* stream) {
   HH_GUARD_BEGIN
   if (!dec) return fail(-1, "hh_decoder_forward: null handle");
-  return dec->impl.forward(features, stride_b, stride_row, B, T, hs, logits, boxes, S(stream));
+  return dec->impl.forward(features, false, stride_b, stride_row, B, T, hs, logits, boxes, S(stream));
+  HH_GUARD_END
+}
+int hh_decoder_forward_bf16(hh_decoder* dec, const void* features, int64_t stride_b, int64_t stride_row, int B, int T,
+                            float* hs, float* logits, float* boxes, void* stream) {
+  HH_GUARD_BEGIN
+  if (!dec) return fail(-1, "hh_decoder_forward_bf16: null handle");
+  return dec->impl.forward(features, true, stride_b, stride_row, B, T, hs, logits, boxes, S(stream));
   HH_GUARD_END
 }
 int hh_decoder_forward_train(hh_decoder* dec, const float* features, int64_t stride_b, int64_t stride_row, int B, int T,
                              float* hs, float* logits, float* boxes, void* stream) {
   HH_GUARD_BEGIN
   if (!dec) return fail(-1, "hh_decoder_forward_train: null handle");
-  return dec->impl.forward(features, stride_b, stride_row, B, T, hs, logits, boxes, S(stream), true);
+  return dec->impl.forward(features, false, stride_b, stride_row, B, T, hs, logits, boxes, S(stream), true);
+  HH_GUARD_END
+}
+int hh_decoder_forward_train_bf16(hh_decoder* dec, const void* features, int64_t stride_b, int64_t stride_row, int B,
+                                  int T, float* hs, float* logits, float* boxes, void* stream) {
+  HH_GUARD_BEGIN
+  if (!dec) return fail(-1, "hh_decoder_forward_train_bf16: null handle");
+  return dec->impl.forward(features, true, stride_b, stride_row, B, T, hs, logits, boxes, S(stream), true);
   HH_GUARD_END
 }
 int hh_decoder_set_dropout(hh_decoder* dec, float p, uint64_t seed, uint32_t offset) {

@@ -221,20 +221,21 @@ int Encoder::pack(cudaStream_t s) {
   return 0;
 }
 
-int Encoder::forward(const float* video, int B, int nblocks, float* fmap, cudaStream_t s) {
+int Encoder::forward(const float* video, int B, int nblocks, const Fmap& out, cudaStream_t s) {
   HH_REQUIRE(video != nullptr, "encoder forward: null buffer");
-  return run(video, nullptr, nullptr, nullptr, B, nblocks, fmap, s);
+  return run(video, nullptr, nullptr, nullptr, B, nblocks, out, s);
 }
 
-int Encoder::forward_u8(const uint8_t* frames, const float* mean, const float* stdv, int B, float* fmap, cudaStream_t s) {
+int Encoder::forward_u8(const uint8_t* frames, const float* mean, const float* stdv, int B, const Fmap& out, cudaStream_t s) {
   HH_REQUIRE(frames != nullptr && mean != nullptr && stdv != nullptr, "encoder forward_u8: null buffer");
-  return run(nullptr, frames, mean, stdv, B, -1, fmap, s);
+  return run(nullptr, frames, mean, stdv, B, -1, out, s);
 }
 
 int Encoder::run(const float* video, const uint8_t* frames, const float* mean, const float* stdv, int B, int nblocks,
-                 float* fmap, cudaStream_t s) {
+                 const Fmap& out, cudaStream_t s) {
   HH_REQUIRE(B > 0, "encoder forward: empty batch");
-  HH_REQUIRE(fmap != nullptr, "encoder forward: null buffer");
+  HH_REQUIRE((out.f32 != nullptr) != (out.b16 != nullptr), "encoder forward: exactly one feature-map buffer");
+  HH_REQUIRE(out.cls == nullptr || out.b16 != nullptr, "encoder forward: the CLS buffer goes with the bf16 map");
   if (weights.dirty) RC(pack(s));
   if (nblocks < 0 || nblocks > cfg.depth) nblocks = cfg.depth;
   launches = 0;
@@ -268,6 +269,12 @@ int Encoder::run(const float* video, const uint8_t* frames, const float* mean, c
     const int Bc = (B - b0) < chunk ? (B - b0) : chunk;
     const int M = Bc * N;
     const int P = Bc * T * n;
+    // this chunk's rows of the final norm's outputs (fp32 map, or bf16 map + fp32 CLS rows)
+    LnArgs fin{};
+    fin.out_f32 = out.f32 ? out.f32 + static_cast<size_t>(b0) * N * D : nullptr;
+    fin.out_bf16 = out.b16 ? out.b16 + static_cast<size_t>(b0) * N * D : nullptr;
+    fin.cls_f32 = out.cls ? out.cls + static_cast<size_t>(b0) * D : nullptr;
+    fin.cls_mod = N;
     // patch embed (LaviLa.py:218-223,540-542) + CLS/pos/temporal + ln_pre (:545-559)
     if (frames) {
       PROF(K_EMBED, im2col_patches_u8(frames + static_cast<size_t>(b0) * T * frame_elems, mean, stdv, patches, Bc * T,
@@ -279,7 +286,7 @@ int Encoder::run(const float* video, const uint8_t* frames, const float* mean, c
     PROF(K_GEMM_PATCH, gemm_bf16(patches, Kp, static_cast<const bf16*>(w_patch.ptr), Kp, tok, D, nullptr, nullptr, 0, P, D,
                                  Kp, EPI_BIAS_F32, s));
     if (fused_ln) {
-      RC(run_blocks_fused(tok, Bc, nblocks, fmap + static_cast<size_t>(b0) * N * D, s));
+      RC(run_blocks_fused(tok, Bc, nblocks, fin, s));
       continue;
     }
     PROF(K_EMBED, assemble_tokens_ln(tok, weights.get("cls_token"), weights.get("pos_embed"), weights.get("temporal_embed"),
@@ -291,7 +298,7 @@ int Encoder::run(const float* video, const uint8_t* frames, const float* mean, c
     const bf16* pending = nullptr;
     const bf16* pending2 = nullptr;
     auto ln_fused = [&](const bf16* delta, const bf16* delta2, bool write_x, const std::string& nm, float eps,
-                        bf16* out16, float* out32) {
+                        bf16* out16, float* out32, float* cls32 = nullptr) {
       LnArgs ln{};
       ln.x = x;
       ln.ldx = D;
@@ -303,6 +310,8 @@ int Encoder::run(const float* video, const uint8_t* frames, const float* mean, c
       ln.eps = eps;
       ln.out_bf16 = out16;
       ln.out_f32 = out32;
+      ln.cls_f32 = cls32;
+      ln.cls_mod = N;
       ln.M = M;
       ln.D = D;
       prof.begin(K_LN, s);
@@ -338,7 +347,7 @@ int Encoder::run(const float* video, const uint8_t* frames, const float* mean, c
       pending2 = dl;
       launches += 3;
     }
-    RC(ln_fused(pending, pending2, false, "norm", 1e-6f, nullptr, fmap + static_cast<size_t>(b0) * N * D));
+    RC(ln_fused(pending, pending2, false, "norm", 1e-6f, fin.out_bf16, fin.out_f32, fin.cls_f32));
     launches += 1;
   }
   return 0;
@@ -353,7 +362,7 @@ int Encoder::run(const float* video, const uint8_t* frames, const float* mean, c
 //   h     = QuickGELU(Linear'(z, stats))               norm2 folded into mlp.fc1              (:388)
 //   x, z  = x + fc2(h), stats                                                                 (:388)
 // x moves 26 bytes per element per layer (3 reads, 2 writes, 3 bf16 copies) instead of 36, in 8 launches instead of 11.
-int Encoder::run_blocks_fused(const float* tok, int Bc, int nblocks, float* fmap_out, cudaStream_t s) {
+int Encoder::run_blocks_fused(const float* tok, int Bc, int nblocks, LnArgs& ln, cudaStream_t s) {
   const int T = cfg.num_frames, D = cfg.embed_dim, H = cfg.num_heads, Hd = cfg.mlp_hidden;
   const int M = Bc * N;
   float* x = static_cast<float*>(ws_x.ptr);
@@ -399,13 +408,12 @@ int Encoder::run_blocks_fused(const float* tok, int Bc, int nblocks, float* fmap
     PROF(K_GEMM_FC2, produce(h, Hd, L.w_fc2, weights.get(p + "mlp.fc2.bias"), true));
     launches += 8;
   }
-  LnArgs ln{};
+  // final norm into the outputs the caller set in `ln`
   ln.x = x;
   ln.ldx = D;
   ln.w = weights.get("norm.weight");
   ln.b = weights.get("norm.bias");
   ln.eps = 1e-6f;
-  ln.out_f32 = fmap_out;
   ln.M = M;
   ln.D = D;
   PROF(K_LN, layernorm_rows(ln, s));
@@ -553,8 +561,8 @@ static int lin(const float* in, int ldi, const float* in_add, int add_mod, const
   return linear_f32(la, s);
 }
 
-int Decoder::forward(const float* features, int64_t stride_b, int64_t stride_row, int B, int T, float* hs, float* logits,
-                     float* boxes, cudaStream_t s, bool save) {
+int Decoder::forward(const void* features, bool feat_bf16, int64_t stride_b, int64_t stride_row, int B, int T, float* hs,
+                     float* logits, float* boxes, cudaStream_t s, bool save) {
   HH_REQUIRE(B > 0 && features && hs && logits && boxes, "decoder forward: bad arguments");
   HH_REQUIRE(T == cfg.num_frames, "decoder forward: T must equal num_frames (construct_3d_pos_embed, tfm_decoder.py:161-166)");
   if (weights.dirty) RC(pack(s));
@@ -564,7 +572,15 @@ int Decoder::forward(const float* features, int64_t stride_b, int64_t stride_row
   const int n = cfg.patches_per_frame, S = T * n, heads = cfg.nhead, ncls = cfg.num_classes1;
   const int R = B * Q;
   const size_t BS = static_cast<size_t>(B) * S;
-  RC(ws_feat.reserve(BS * F * 2));
+  // Direct path (inference, bf16 map): the proj GEMM reads A from the caller's rows, clip b's S patch rows starting at
+  // row b * pitch (pitch = stride_b / stride_row: image_feature_map[:, 1:] skips each clip's CLS row).  TMA needs 16-byte
+  // rows and segments of whole 128-row tiles.  Every other case gathers the rows into ws_feat first; the training
+  // forward always does, because backward() reads that copy (the caller may reuse its tensor before backward()).
+  const int64_t pitch = (B == 1) ? S : (stride_row > 0 ? stride_b / stride_row : 0);
+  const bool direct = feat_bf16 && !save && S % 128 == 0 && (reinterpret_cast<uintptr_t>(features) & 15) == 0 &&
+                      stride_row > 0 && stride_row % 8 == 0 && (B == 1 || (stride_b % stride_row == 0 && pitch >= S)) &&
+                      stride_row <= 0x7fffffff && pitch <= 0x7fffffff;
+  if (!direct) RC(ws_feat.reserve(BS * F * 2));
   RC(ws_memf.reserve(BS * C * 4));
   RC(ws_mem.reserve(BS * C * 2));
   RC(ws_mempos.reserve(BS * C * 2));
@@ -621,9 +637,18 @@ int Decoder::forward(const float* features, int64_t stride_b, int64_t stride_row
   if (save) saved_drop = dr;
 
   // proj (no bias, :200) -> pre_norm (:86) ; memory and memory+pos in bf16 for the K/V GEMMs
-  PROF(K_DEC_GEMM, cast_rows_bf16(features, stride_b, stride_row, S, feat, static_cast<int>(BS), F, s));
-  PROF(K_DEC_GEMM, gemm_bf16(feat, F, static_cast<const bf16*>(w_proj.ptr), F, memf, C, nullptr, nullptr, 0, static_cast<int>(BS), C, F,
-               EPI_BIAS_F32, s));
+  if (direct) {
+    PROF(K_DEC_GEMM, gemm_bf16_rowseg(static_cast<const bf16*>(features), static_cast<int>(stride_row), S, static_cast<int>(pitch),
+                                      static_cast<const bf16*>(w_proj.ptr), F, memf, C, nullptr, static_cast<int>(BS), C, F,
+                                      EPI_BIAS_F32, s));
+  } else {
+    if (feat_bf16)
+      PROF(K_DEC_GEMM, cast_rows_bf16(static_cast<const bf16*>(features), stride_b, stride_row, S, feat, static_cast<int>(BS), F, s));
+    else
+      PROF(K_DEC_GEMM, cast_rows_bf16(static_cast<const float*>(features), stride_b, stride_row, S, feat, static_cast<int>(BS), F, s));
+    PROF(K_DEC_GEMM, gemm_bf16(feat, F, static_cast<const bf16*>(w_proj.ptr), F, memf, C, nullptr, nullptr, 0, static_cast<int>(BS), C,
+                               F, EPI_BIAS_F32, s));
+  }
   LnArgs ln{};
   ln.x = memf; ln.ldx = C;
   ln.w = weights.get("transformer.pre_norm.weight"); ln.b = weights.get("transformer.pre_norm.bias"); ln.eps = 1e-5f;
@@ -636,7 +661,7 @@ int Decoder::forward(const float* features, int64_t stride_b, int64_t stride_row
   PROF(K_DEC_GEMM, gemm_bf16(mem, C, static_cast<const bf16*>(w_vall.ptr), C, Vall, Lr * C, static_cast<const float*>(b_vall.ptr), nullptr,
                0, static_cast<int>(BS), Lr * C, C, EPI_BIAS_BF16, s));
   HH_CHECK_CUDA(cudaMemsetAsync(tgt, 0, static_cast<size_t>(R) * C * 4, s));  // tgt = zeros (:84)
-  launches += 6;
+  launches += direct ? 5 : 6;
 
   auto lnq = [&](const float* x, const std::string& nm, float* out) {
     LnArgs a{};

@@ -73,15 +73,22 @@ struct Encoder {
   explicit Encoder(const hh_encoder_cfg& c);
   static int validate(const hh_encoder_cfg& c);
   int pack(cudaStream_t s);
-  int forward(const float* video, int B, int nblocks, float* fmap, cudaStream_t s);
+  // The feature map leaves the final norm as fp32 (Fmap::f32) or as bf16 (Fmap::b16, with the CLS rows also written in
+  // fp32 to Fmap::cls [B, D] when it is set: the same values as the fp32 map's rows b * N).
+  struct Fmap {
+    float* f32 = nullptr;
+    bf16* b16 = nullptr;
+    float* cls = nullptr;
+  };
+  int forward(const float* video, int B, int nblocks, const Fmap& out, cudaStream_t s);
   // raw frames uint8 [B,T,H,W,3] with the loader's /255 + mean/std normalisation fused into the patch loader
-  int forward_u8(const uint8_t* frames, const float* mean, const float* stdv, int B, float* fmap, cudaStream_t s);
+  int forward_u8(const uint8_t* frames, const float* mean, const float* stdv, int B, const Fmap& out, cudaStream_t s);
   double flops_per_clip() const;
 
  private:
-  int run(const float* video, const uint8_t* frames, const float* mean, const float* stdv, int B, int nblocks, float* fmap,
-          cudaStream_t s);
-  int run_blocks_fused(const float* tok, int Bc, int nblocks, float* fmap_out, cudaStream_t s);
+  int run(const float* video, const uint8_t* frames, const float* mean, const float* stdv, int B, int nblocks,
+          const Fmap& out, cudaStream_t s);
+  int run_blocks_fused(const float* tok, int Bc, int nblocks, LnArgs& final_norm, cudaStream_t s);
 
  public:
 };
@@ -122,9 +129,10 @@ struct Decoder {
   ~Decoder();
   static int validate(const hh_decoder_cfg& c);
   int pack(cudaStream_t s);
-  // save = true keeps every layer's activations for backward() (training forward; dropout per next_drop)
-  int forward(const float* features, int64_t stride_b, int64_t stride_row, int B, int T, float* hs, float* logits,
-              float* boxes, cudaStream_t s, bool save = false);
+  // save = true keeps every layer's activations for backward() (training forward; dropout per next_drop).
+  // features: fp32, or bf16 when feat_bf16; inference reads a suitably laid out bf16 map in place (no ws_feat copy)
+  int forward(const void* features, bool feat_bf16, int64_t stride_b, int64_t stride_row, int B, int T, float* hs,
+              float* logits, float* boxes, cudaStream_t s, bool save = false);
   // Gradients of all decoder parameters for upstream d_hs [L,B,Q,C] and d_boxes [L,B*Tb,Q,4] (either may be null = 0);
   // hs / boxes are the outputs of the matching forward(save = true).  Results are read with grad().
   int backward(const float* hs, const float* boxes, const float* d_hs, const float* d_boxes, cudaStream_t s);

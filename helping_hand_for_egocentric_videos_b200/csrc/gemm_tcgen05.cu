@@ -88,6 +88,8 @@ struct GemmArgs {
   // EPI_RES_STATS_BF16: per-row partials of the rows this GEMM writes, [tiles_n][M][2]; write the fp32 sum back in place
   float* stats_out;
   int writeback;
+  // segmented A rows (gemm_bf16_rowseg): logical row m is A row m + (m / a_seg_rows) * a_seg_skip; 0 = contiguous
+  int a_seg_rows, a_seg_skip;
 };
 
 __device__ __forceinline__ float quick_gelu(float x) {
@@ -231,13 +233,17 @@ gemm_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constant__ C
         const int mp = tile / p.tiles_n;
         const int n_blk = tile - mp * p.tiles_n;
         const int m_blk = CLUSTER ? 2 * mp + cta_rank : mp;
+        // A row of this tile: a 128-row box never straddles two segments (a_seg_rows % 128 == 0); a pair's padding tile
+        // past M maps past the end of A as well and is zero-filled, as without segments
+        int a_row = m_blk * BLOCK_M;
+        if (p.a_seg_rows) a_row += (a_row / p.a_seg_rows) * p.a_seg_skip;
         for (int kb = 0; kb < num_kb; ++kb) {
           { TR_T0(); mbar_wait(&empty_bar[stage], phase ^ 1u); TR_ADD(1); }
           uint8_t* sa = stage_base + stage * C::STAGE_BYTES;
           uint8_t* sb = sa + C::A_BYTES;
           if constexpr (TWOSM) {  // my A rows + my half of the W tile, into MY smem, signalled on the leader's barrier
             if (cta_rank == 0) mbar_arrive_expect_tx(&full_bar[stage], 2 * C::STAGE_BYTES);
-            tma_load_2d_2sm(&tma_a, &full_bar[stage], sa, kb * BLOCK_K, m_blk * BLOCK_M);
+            tma_load_2d_2sm(&tma_a, &full_bar[stage], sa, kb * BLOCK_K, a_row);
             tma_load_2d_2sm(&tma_b, &full_bar[stage], sb, kb * BLOCK_K, n_blk * BLOCK_N + cta_rank * (BLOCK_N / 2));
             if (++stage == C::STAGES) {
               stage = 0;
@@ -246,7 +252,7 @@ gemm_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constant__ C
             continue;
           }
           mbar_arrive_expect_tx(&full_bar[stage], C::STAGE_BYTES);
-          tma_load_2d(&tma_a, &full_bar[stage], sa, kb * BLOCK_K, m_blk * BLOCK_M);
+          tma_load_2d(&tma_a, &full_bar[stage], sa, kb * BLOCK_K, a_row);
           if constexpr (CLUSTER) {  // my half of the W tile, into both CTAs (box = BLOCK_N/2 rows)
             tma_load_2d_mcast(&tma_b, &full_bar[stage], sb + cta_rank * (C::B_BYTES / 2), kb * BLOCK_K,
                               n_blk * BLOCK_N + cta_rank * (BLOCK_N / 2), static_cast<uint16_t>(3));
@@ -842,9 +848,9 @@ extern "C" int hh_debug_gemm_trace(unsigned long long* out, int n) {
 
 int gemm_stats_parts(int M, int N) { return plan_tiles(M, N, EPI_RES_STATS_BF16, true).tiles_n; }
 
-int gemm_bf16_fused(const bf16* A, int lda, const bf16* W, int ldw, void* out, int ldc, const float* bias,
-                    float* residual, int ldr, int M, int N, int K, int epilogue, const GemmFuse& fuse,
-                    cudaStream_t stream) {
+static int gemm_impl(const bf16* A, int lda, int seg_rows, int seg_pitch, const bf16* W, int ldw, void* out, int ldc,
+                     const float* bias, float* residual, int ldr, int M, int N, int K, int epilogue, const GemmFuse& fuse,
+                     cudaStream_t stream) {
   HH_REQUIRE(M > 0 && N > 0 && K > 0, "gemm_bf16: empty problem");
   HH_REQUIRE(lda % 8 == 0 && ldw % 8 == 0, "gemm_bf16: lda/ldw must be multiples of 8 elements (16-byte TMA strides)");
   HH_REQUIRE(K % 8 == 0, "gemm_bf16: K must be a multiple of 8");
@@ -873,10 +879,18 @@ int gemm_bf16_fused(const bf16* A, int lda, const bf16* W, int ldw, void* out, i
     HH_REQUIRE((reinterpret_cast<uintptr_t>(residual) & 15) == 0 && ldr % 4 == 0,
                "gemm_bf16: residual must be 16-byte aligned with a 16-byte multiple row pitch");
   }
+  int a_rows = M;   // rows A's tensor map covers
+  if (seg_rows > 0) {
+    HH_REQUIRE(seg_rows % BLOCK_M == 0 && M % seg_rows == 0 && seg_pitch >= seg_rows,
+               "gemm_bf16_rowseg: segments must be whole 128-row tiles, M a whole number of segments, pitch >= rows");
+    const long long span = static_cast<long long>(M / seg_rows - 1) * seg_pitch + seg_rows;
+    HH_REQUIRE(span <= 0x7fffffffLL, "gemm_bf16_rowseg: A spans too many rows");
+    a_rows = static_cast<int>(span);
+  }
   const TilePlan t = plan_tiles(M, N, epilogue, tma_store);
   const int bn = t.bn;
   CUtensorMap ta, tb, tc, tr;
-  int rc = make_tmap(&ta, A, M, K, lda, BLOCK_M);
+  int rc = make_tmap(&ta, A, a_rows, K, lda, BLOCK_M);
   if (rc) return rc;
   rc = make_tmap(&tb, W, N, K, ldw, t.cluster ? bn / 2 : bn);
   if (rc) return rc;
@@ -911,8 +925,23 @@ int gemm_bf16_fused(const bf16* A, int lda, const bf16* W, int ldw, void* out, i
   args.eps = fuse.eps;
   args.stats_out = fuse.stats_out;
   args.writeback = fuse.writeback;
+  args.a_seg_rows = seg_rows > 0 ? seg_rows : 0;
+  args.a_seg_skip = seg_rows > 0 ? seg_pitch - seg_rows : 0;
   if (bn == 256) return dispatch_epi<256>(ta, tb, tc, tr, tma_store, t.cluster, t.twosm, args, epilogue, stream);
   return dispatch_epi<128>(ta, tb, tc, tr, tma_store, t.cluster, false, args, epilogue, stream);
+}
+
+int gemm_bf16_fused(const bf16* A, int lda, const bf16* W, int ldw, void* out, int ldc, const float* bias,
+                    float* residual, int ldr, int M, int N, int K, int epilogue, const GemmFuse& fuse,
+                    cudaStream_t stream) {
+  return gemm_impl(A, lda, 0, 0, W, ldw, out, ldc, bias, residual, ldr, M, N, K, epilogue, fuse, stream);
+}
+
+int gemm_bf16_rowseg(const bf16* A, int lda, int seg_rows, int seg_pitch, const bf16* W, int ldw, void* out, int ldc,
+                     const float* bias, int M, int N, int K, int epilogue, cudaStream_t stream) {
+  HH_REQUIRE(epilogue == EPI_BIAS_BF16 || epilogue == EPI_BIAS_F32, "gemm_bf16_rowseg: plain bias epilogues only");
+  HH_REQUIRE(seg_rows > 0, "gemm_bf16_rowseg: seg_rows must be positive");
+  return gemm_impl(A, lda, seg_rows, seg_pitch, W, ldw, out, ldc, bias, nullptr, 0, M, N, K, epilogue, GemmFuse{}, stream);
 }
 
 int gemm_bf16(const bf16* A, int lda, const bf16* W, int ldw, void* out, int ldc, const float* bias,

@@ -70,6 +70,12 @@ int gemm_bf16_fused(const bf16* A, int lda, const bf16* W, int ldw, void* out, i
 // C[M,N] = epilogue(A[M,K] * W[N,K]^T); A, W bf16 with K contiguous. bias fp32 [N] or nullptr.
 int gemm_bf16(const bf16* A, int lda, const bf16* W, int ldw, void* out, int ldc, const float* bias,
               const float* residual, int ldr, int M, int N, int K, int epilogue, cudaStream_t stream);
+// gemm_bf16 (EPI_BIAS_BF16 / EPI_BIAS_F32) over A rows in segments: logical row m is row m + (m / seg_rows) *
+// (seg_pitch - seg_rows) of A (row stride lda), i.e. M / seg_rows segments of seg_rows rows that start seg_pitch rows
+// apart (per-clip patch rows of a feature map whose CLS rows are skipped).  seg_rows % 128 == 0 (every 128-row tile
+// lies in one segment), M % seg_rows == 0, seg_pitch >= seg_rows.
+int gemm_bf16_rowseg(const bf16* A, int lda, int seg_rows, int seg_pitch, const bf16* W, int ldw, void* out, int ldc,
+                     const float* bias, int M, int N, int K, int epilogue, cudaStream_t stream);
 
 // ---------------------------------------------------------------- row-wise kernels (rows.cu)
 // y = LayerNorm(x (+ add_rows_mod)) * w + b.  x fp32 [M, D] (row stride ldx). Outputs (any may be null):
@@ -84,11 +90,14 @@ struct LnArgs {
   const float* post_add; int post_mod;   // optional positional term added after the norm
   float* out2_f32; bf16* out2_bf16;
   int M, D;
+  float* cls_f32; int cls_mod;   // optional fp32 [M / cls_mod, D]: rows with row % cls_mod == 0 also go here (CLS rows)
 };
 int layernorm_rows(const LnArgs& a, cudaStream_t stream);
 
-// fp32 (strided rows) -> bf16 contiguous [rows, cols]: row r = (r / inner) * outer_stride + (r % inner) * row_stride.
+// fp32 or bf16 (strided rows) -> bf16 contiguous [rows, cols]: row r = (r / inner) * outer_stride + (r % inner) * row_stride.
 int cast_rows_bf16(const float* src, long long outer_stride, long long row_stride, int inner, bf16* dst, int rows,
+                   int cols, cudaStream_t stream);
+int cast_rows_bf16(const bf16* src, long long outer_stride, long long row_stride, int inner, bf16* dst, int rows,
                    int cols, cudaStream_t stream);
 
 // ---------------------------------------------------------------- encoder satellites (embed.cu)

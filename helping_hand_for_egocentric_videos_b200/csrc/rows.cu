@@ -79,6 +79,7 @@ __global__ void __launch_bounds__(256) ln_rows_kernel(const LnArgs a) {
   const float rstd = rsqrtf(warp_sum(ss) / static_cast<float>(a.D) + a.eps);
   const size_t orow = static_cast<size_t>(warp) * a.D;
   const float* padd = a.post_add ? a.post_add + static_cast<size_t>(warp % a.post_mod) * a.D : nullptr;
+  float* const crow = (a.cls_f32 && warp % a.cls_mod == 0) ? a.cls_f32 + static_cast<size_t>(warp / a.cls_mod) * a.D : nullptr;
 #pragma unroll
   for (int j = 0; j < LN_MAX_VEC; ++j) {
     if (j < nv) {
@@ -91,6 +92,7 @@ __global__ void __launch_bounds__(256) ln_rows_kernel(const LnArgs a) {
       y.z = v[j].z * rstd * w.z + b.z;
       y.w = v[j].w * rstd * w.w + b.w;
       if (a.out_f32) *reinterpret_cast<float4*>(a.out_f32 + orow + c) = y;
+      if (crow) *reinterpret_cast<float4*>(crow + c) = y;
       if (a.out_bf16) {
         uint2 pk = make_uint2(pack_bf16x2(y.x, y.y), pack_bf16x2(y.z, y.w));
         *reinterpret_cast<uint2*>(a.out_bf16 + orow + c) = pk;
@@ -108,7 +110,15 @@ __global__ void __launch_bounds__(256) ln_rows_kernel(const LnArgs a) {
   }
 }
 
-__global__ void __launch_bounds__(256) cast_rows_kernel(const float* __restrict__ src, long long outer_stride,
+// 4 columns per step: float4 -> packed bf16 (fp32 rows) or a plain 8-byte copy (bf16 rows, the gather alone)
+__device__ __forceinline__ uint2 load4_bf16(const float* s) {
+  const float4 v = *reinterpret_cast<const float4*>(s);
+  return make_uint2(pack_bf16x2(v.x, v.y), pack_bf16x2(v.z, v.w));
+}
+__device__ __forceinline__ uint2 load4_bf16(const bf16* s) { return *reinterpret_cast<const uint2*>(s); }
+
+template <typename Src>
+__global__ void __launch_bounds__(256) cast_rows_kernel(const Src* __restrict__ src, long long outer_stride,
                                                         long long row_stride, int inner, bf16* __restrict__ dst,
                                                         int rows, int cols) {
   const int vec_per_row = cols >> 2;
@@ -117,10 +127,8 @@ __global__ void __launch_bounds__(256) cast_rows_kernel(const float* __restrict_
        i += static_cast<long long>(gridDim.x) * blockDim.x) {
     const int r = static_cast<int>(i / vec_per_row);
     const int c = static_cast<int>(i - static_cast<long long>(r) * vec_per_row) * 4;
-    const float* s = src + (r / inner) * outer_stride + (r % inner) * row_stride + c;
-    const float4 v = *reinterpret_cast<const float4*>(s);
-    *reinterpret_cast<uint2*>(dst + static_cast<size_t>(r) * cols + c) =
-        make_uint2(pack_bf16x2(v.x, v.y), pack_bf16x2(v.z, v.w));
+    const Src* s = src + (r / inner) * outer_stride + (r % inner) * row_stride + c;
+    *reinterpret_cast<uint2*>(dst + static_cast<size_t>(r) * cols + c) = load4_bf16(s);
   }
 }
 
@@ -283,17 +291,29 @@ int layernorm_rows(const LnArgs& a, cudaStream_t stream) {
   return 0;
 }
 
-int cast_rows_bf16(const float* src, long long outer_stride, long long row_stride, int inner, bf16* dst, int rows,
-                   int cols, cudaStream_t stream) {
+template <typename Src>
+static int cast_rows_impl(const Src* src, long long outer_stride, long long row_stride, int inner, bf16* dst, int rows,
+                          int cols, cudaStream_t stream) {
   HH_REQUIRE(rows > 0 && cols > 0 && cols % 4 == 0, "cast_rows_bf16: cols must be a multiple of 4");
-  HH_REQUIRE(outer_stride % 4 == 0 && row_stride % 4 == 0, "cast_rows_bf16: strides must keep 16-byte alignment");
+  HH_REQUIRE(outer_stride % 4 == 0 && row_stride % 4 == 0, "cast_rows_bf16: strides must keep 4-element alignment");
+  HH_REQUIRE((reinterpret_cast<uintptr_t>(src) & (4 * sizeof(Src) - 1)) == 0, "cast_rows_bf16: misaligned source");
   const long long total = static_cast<long long>(rows) * (cols / 4);
   long long blocks = (total + 255) / 256;
   const long long cap = static_cast<long long>(num_sms()) * 16;
   if (blocks > cap) blocks = cap;
-  cast_rows_kernel<<<static_cast<int>(blocks), 256, 0, stream>>>(src, outer_stride, row_stride, inner, dst, rows, cols);
+  cast_rows_kernel<Src><<<static_cast<int>(blocks), 256, 0, stream>>>(src, outer_stride, row_stride, inner, dst, rows, cols);
   HH_CHECK_LAUNCH("cast_rows_kernel");
   return 0;
+}
+
+int cast_rows_bf16(const float* src, long long outer_stride, long long row_stride, int inner, bf16* dst, int rows,
+                   int cols, cudaStream_t stream) {
+  return cast_rows_impl(src, outer_stride, row_stride, inner, dst, rows, cols, stream);
+}
+
+int cast_rows_bf16(const bf16* src, long long outer_stride, long long row_stride, int inner, bf16* dst, int rows,
+                   int cols, cudaStream_t stream) {
+  return cast_rows_impl(src, outer_stride, row_stride, inner, dst, rows, cols, stream);
 }
 
 int f32_to_bf16(const float* src, bf16* dst, size_t n, cudaStream_t stream) {

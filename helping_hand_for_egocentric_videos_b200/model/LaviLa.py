@@ -194,6 +194,20 @@ class SpaceTimeTransformer(_DirtyHooks, nn.Module):
         self._cfg = L.EncoderCfg(img_size, patch_size, num_frames, embed_dim, depth, num_heads, int(embed_dim * mlp_ratio))
         self._handle = None
         self._sync = _ParamSync()
+        self.feature_map_dtype = torch.float32
+
+    @property
+    def feature_map_dtype(self):
+        """dtype of the feature map forward_features returns: torch.float32 (default) or torch.bfloat16.  The bf16 map
+        is the fp32 one rounded to nearest-even at half the bytes; x_cls stays fp32 and bit-identical, and ObjDecoder
+        gives the same outputs on either map (it rounds its input to bf16 itself)."""
+        return self._feature_map_dtype
+
+    @feature_map_dtype.setter
+    def feature_map_dtype(self, dtype):
+        if dtype not in (torch.float32, torch.bfloat16):
+            raise ValueError("feature_map_dtype must be torch.float32 or torch.bfloat16, got %r" % (dtype,))
+        self._feature_map_dtype = dtype
 
     # -- engine plumbing ---------------------------------------------------------------------------------------
     def _engine(self):
@@ -268,7 +282,8 @@ class SpaceTimeTransformer(_DirtyHooks, nn.Module):
     @torch.no_grad()
     def forward_features(self, x, use_checkpoint=False, cls_at_last=True, _nblocks=-1):
         """x [B,T,3,H,W] -> (x_cls [B,D], fmap [B,1+T*n,D]); the tower is frozen in every reference script
-        (run/train.py:109 runs it under no_grad), so no autograd graph is recorded."""
+        (run/train.py:109 runs it under no_grad), so no autograd graph is recorded.  fmap has feature_map_dtype
+        (x_cls is fp32 either way); the `_nblocks` test hook always returns fp32."""
         if not x.is_cuda:
             raise RuntimeError("SpaceTimeTransformer (B200): input is on %s; there is no CPU fallback" % x.device)
         b, t, c, hh, ww = x.shape
@@ -281,6 +296,12 @@ class SpaceTimeTransformer(_DirtyHooks, nn.Module):
         self.sync_weights()
         x = x.float().contiguous()
         n_tok = 1 + t * self.patches_per_frame
+        if self.feature_map_dtype == torch.bfloat16 and _nblocks == -1:     # the truncated-forward hook stays fp32
+            fmap = torch.empty(b, n_tok, self.embed_dim, dtype=torch.bfloat16, device=x.device)
+            cls = torch.empty(b, self.embed_dim, dtype=torch.float32, device=x.device)
+            L.check(L.load().hh_encoder_forward_bf16(self._engine(), L.ptr(x), b, L.ptr(fmap), L.ptr(cls), L.stream_ptr()),
+                    "hh_encoder_forward_bf16")
+            return self.pre_logits(cls), fmap
         fmap = torch.empty(b, n_tok, self.embed_dim, dtype=torch.float32, device=x.device)
         L.check(L.load().hh_encoder_forward_n(self._engine(), L.ptr(x), b, _nblocks, L.ptr(fmap), L.stream_ptr()),
                 "hh_encoder_forward")
@@ -307,7 +328,14 @@ class SpaceTimeTransformer(_DirtyHooks, nn.Module):
         frames = frames.contiguous()
         mean = (C.c_float * 3)(*[float(v) for v in norm_mean])
         std = (C.c_float * 3)(*[float(v) for v in norm_std])
-        fmap = torch.empty(b, 1 + t * self.patches_per_frame, self.embed_dim, dtype=torch.float32, device=frames.device)
+        n_tok = 1 + t * self.patches_per_frame
+        if self.feature_map_dtype == torch.bfloat16:
+            fmap = torch.empty(b, n_tok, self.embed_dim, dtype=torch.bfloat16, device=frames.device)
+            cls = torch.empty(b, self.embed_dim, dtype=torch.float32, device=frames.device)
+            L.check(L.load().hh_encoder_forward_u8_bf16(self._engine(), L.ptr(frames), b, mean, std, L.ptr(fmap), L.ptr(cls),
+                                                        L.stream_ptr()), "hh_encoder_forward_u8_bf16")
+            return self.pre_logits(cls), fmap
+        fmap = torch.empty(b, n_tok, self.embed_dim, dtype=torch.float32, device=frames.device)
         L.check(L.load().hh_encoder_forward_u8(self._engine(), L.ptr(frames), b, mean, std, L.ptr(fmap), L.stream_ptr()),
                 "hh_encoder_forward_u8")
         return self.pre_logits(fmap[:, 0]), fmap

@@ -318,7 +318,11 @@ class ObjDecoder(_DirtyHooks, nn.Module):
         hs = torch.empty(L_, B, Q, Cd, dtype=torch.float32, device=dev)
         logits = torch.empty(L_, B * (4 if traj else 1), Q, ncls, dtype=torch.float32, device=dev)
         boxes = torch.empty(L_, B * (T if traj else 1), Q, 4, dtype=torch.float32, device=dev)
-        fn = L.load().hh_decoder_forward_train if train else L.load().hh_decoder_forward
+        lib = L.load()
+        if features.dtype == torch.bfloat16:
+            fn = lib.hh_decoder_forward_train_bf16 if train else lib.hh_decoder_forward_bf16
+        else:
+            fn = lib.hh_decoder_forward_train if train else lib.hh_decoder_forward
         self.last_dropout = None
         if train:
             p = float(self.transformer.dropout_p) if self.training else 0.0
@@ -333,9 +337,11 @@ class ObjDecoder(_DirtyHooks, nn.Module):
         return hs, logits, boxes
 
     def forward(self, features, use_checkpoint=False):
-        """features [B,T,n,F] (fp32, any strides with a unit innermost stride) -> (out, hs, [], []).  With autograd
-        enabled and trainable parameters the engine keeps its activations and the outputs carry the hand-written
-        backward (gradients for every decoder parameter; `features` come from the frozen backbone and get none)."""
+        """features [B,T,n,F] (fp32 or bf16, any strides with a unit innermost stride) -> (out, hs, [], []).  bf16
+        features give the same outputs as their fp32 source (the engine rounds fp32 features to bf16 itself); in eval a
+        bf16 image_feature_map[:, 1:] view is read in place.  With autograd enabled and trainable parameters the engine
+        keeps its activations (and its own copy of the features) and the outputs carry the hand-written backward
+        (gradients for every decoder parameter; `features` come from the frozen backbone and get none)."""
         if not features.is_cuda:
             raise RuntimeError("ObjDecoder (B200): input is on %s; there is no CPU fallback" % features.device)
         B, T, n, F = features.shape
@@ -343,10 +349,11 @@ class ObjDecoder(_DirtyHooks, nn.Module):
             raise RuntimeError("expected features [B,T,%d,%d], got %s" % (self.patches_per_frame, self._cfg.feature_dim,
                                                                           tuple(features.shape)))
         features = features.detach()
-        if features.dtype != torch.float32:
+        if features.dtype not in (torch.float32, torch.bfloat16):
             features = features.float()
-        if features.stride(3) != 1 or features.stride(1) != n * features.stride(2) or features.stride(2) % 4 \
-                or features.stride(0) % 4 or features.data_ptr() % 16:
+        vec = 16 // features.element_size()          # elements per 16 bytes
+        if features.stride(3) != 1 or features.stride(1) != n * features.stride(2) or features.stride(2) % vec \
+                or features.stride(0) % vec or features.data_ptr() % 16:
             features = features.contiguous()
         self.sync_weights()
         params = [p for _, p in self._engine_params()]

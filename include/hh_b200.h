@@ -61,6 +61,14 @@ int hh_encoder_forward_n(hh_encoder* enc, const float* video, int B, int nblocks
  * mean / std: 3 host floats each (per channel, in [0,1] units). */
 int hh_encoder_forward_u8(hh_encoder* enc, const uint8_t* frames, int B, const float* mean, const float* std,
                           float* fmap, void* stream);
+/* The same two forwards with the feature map handed over in bf16: fmap bf16 [B, 1+T*n, D] holds every row of the fp32
+ * map rounded to nearest-even, and cls fp32 [B, D] (may be NULL) receives the CLS rows fmap32[:, 0] unrounded, so x_cls
+ * and the image embedding stay bit-identical to the fp32 entry points.  Half the bytes written and held; the decoder
+ * rounds its input to bf16 anyway, so hh_decoder_forward_bf16 on this map gives what hh_decoder_forward gives on the
+ * fp32 one, bit for bit. */
+int hh_encoder_forward_bf16(hh_encoder* enc, const float* video, int B, void* fmap, float* cls, void* stream);
+int hh_encoder_forward_u8_bf16(hh_encoder* enc, const uint8_t* frames, int B, const float* mean, const float* std,
+                               void* fmap, float* cls, void* stream);
 /* Algorithmic FLOPs of one clip through the encoder (SURVEY.md section 8d formula). */
 double hh_encoder_flops_per_clip(const hh_encoder* enc);
 /* Number of kernel launches issued by the last hh_encoder_forward call. */
@@ -96,6 +104,12 @@ int hh_decoder_set_weight(hh_decoder* dec, const char* key, const float* data, i
  */
 int hh_decoder_forward(hh_decoder* dec, const float* features, int64_t stride_b, int64_t stride_row, int B, int T,
                        float* hs, float* logits, float* boxes, void* stream);
+/* The same forward on bf16 features [B,T,n,F] (same strided layout, strides in elements; rows 8-byte aligned).  When
+ * T*n is a multiple of 128, the rows are 16-byte aligned and stride_b is a multiple of stride_row (image_feature_map[:, 1:]
+ * of a bf16 map qualifies), the first GEMM reads the caller's rows in place: no copy, no feature workspace, one launch
+ * fewer.  Otherwise the rows are first gathered into the engine's workspace. */
+int hh_decoder_forward_bf16(hh_decoder* dec, const void* features, int64_t stride_b, int64_t stride_row, int B, int T,
+                            float* hs, float* logits, float* boxes, void* stream);
 /* Training: the same forward that also keeps every layer's activations inside the engine, then hh_decoder_backward
  * differentiates it.  Dropout of the reference's training mode (nn.Dropout x4 per layer, tfm_decoder.py:372-386, and
  * nn.MultiheadAttention(dropout=p) on the self- and cross-attention probabilities, :365-366) is applied by the training
@@ -108,6 +122,10 @@ int hh_decoder_forward(hh_decoder* dec, const float* features, int64_t stride_b,
  * with hh_decoder_get_grad (fp32, `numel` elements, device memory). */
 int hh_decoder_forward_train(hh_decoder* dec, const float* features, int64_t stride_b, int64_t stride_row, int B, int T,
                              float* hs, float* logits, float* boxes, void* stream);
+/* Training forward on bf16 features.  It always copies the rows into the engine (backward reads that copy), so the
+ * caller may overwrite `features` between this call and hh_decoder_backward. */
+int hh_decoder_forward_train_bf16(hh_decoder* dec, const void* features, int64_t stride_b, int64_t stride_row, int B,
+                                  int T, float* hs, float* logits, float* boxes, void* stream);
 int hh_decoder_set_dropout(hh_decoder* dec, float p, uint64_t seed, uint32_t offset);
 int hh_decoder_backward(hh_decoder* dec, const float* hs, const float* boxes, const float* d_hs, const float* d_boxes,
                         void* stream);
