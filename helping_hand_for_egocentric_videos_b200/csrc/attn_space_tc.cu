@@ -1,6 +1,6 @@
 // Spatial attention on the 5th-generation tensor cores (tcgen05 + TMEM), n <= 256 patches per frame, head dim 64.
-// Same operator as attn_space.cu (VarAttention '(b f) n d', model/LaviLa.py:246-283); that file stays as the
-// mma.sync statement of it (fallback for n > 256 and differential reference).
+// Same operator as attn_space.cu (VarAttention '(b f) n d', model/LaviLa.py:246-283); that file's mma.sync statement of
+// it runs the frames of more than 256 patches.
 //
 // One task = one (clip, frame, head): Q, K, V tiles of [n x 64] bf16.  All n keys fit one accumulator tile, so the
 // softmax is a single exact pass (no online rescaling):
@@ -85,38 +85,13 @@ __device__ __forceinline__ void trace_ev(const TcArgs& p, int role, int it, int 
 
 // tasks are walked from the last (clip, frame, head): those q/k/v rows were written last by the QKV GEMM and are still
 // in L2, and the projection GEMM that follows reads the rows this kernel writes last (the first clips) first
-#ifdef HH_FORWARD_WALK
-#define HH_TASK(t) (t)
-#else
-#define HH_TASK(t) (ntasks - 1 - (t))
-#endif
+__device__ __forceinline__ int task_index(int task, int ntasks) { return ntasks - 1 - task; }
 
 __device__ __forceinline__ void st_shared_v4(uint32_t addr, uint32_t a, uint32_t b, uint32_t c, uint32_t d) {
   asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(addr), "r"(a), "r"(b), "r"(c), "r"(d) : "memory");
 }
 __device__ __forceinline__ uint32_t sw128(uint32_t tile, int row, int chunk) {
   return tile + static_cast<uint32_t>(row * 128 + ((chunk ^ (row & 7)) << 4));
-}
-
-// 2^x for two x <= 0 on the FMA / ALU pipes instead of the MUFU: x = n + f with n = round(x), f in [-0.5, 0.5] (magic-number
-// add), 2^f as a degree-3 polynomial (relative error 7.5e-5, well inside the bf16 rounding of P), n added into the
-// exponent field.  Clamped at -125: 2^-125 is nothing next to a row sum >= 1.
-#ifndef HH_ATTN_EMU
-#define HH_ATTN_EMU 0       // pairs out of every 4 that take this path in the exp pass (0 = all on the MUFU: measured best)
-#endif
-__device__ __forceinline__ float2 poly_exp2x2(float2 x) {
-  const float MAGIC = 12582912.f;   // 1.5 * 2^23
-  x.x = fmaxf(x.x, -125.f);
-  x.y = fmaxf(x.y, -125.f);
-  const float2 xf = __fadd2_rn(x, make_float2(MAGIC, MAGIC));
-  const float2 fl = __fadd2_rn(xf, make_float2(-MAGIC, -MAGIC));
-  const float2 f = __fadd2_rn(x, make_float2(-fl.x, -fl.y));
-  const float c0 = 0.999928074f, c1 = 0.693260986f, c2 = 0.242611122f, c3 = 0.055171667f;
-  float2 q = __ffma2_rn(f, make_float2(c3, c3), make_float2(c2, c2));
-  q = __ffma2_rn(q, f, make_float2(c1, c1));
-  q = __ffma2_rn(q, f, make_float2(c0, c0));
-  return make_float2(__uint_as_float(__float_as_uint(q.x) + (__float_as_uint(xf.x) << 23)),
-                     __uint_as_float(__float_as_uint(q.y) + (__float_as_uint(xf.y) << 23)));
 }
 
 // kFull: n == 256 exactly (the L/14 geometry): no ragged-chunk code in the softmax loops (half the code bytes of the hot
@@ -186,7 +161,7 @@ attn_space_tc_kernel(const __grid_constant__ CUtensorMap tm_in, const __grid_con
       for (int task = blockIdx.x; task < ntasks; task += gridDim.x, ++it) {
         const int st = it & 1;
         const uint32_t ph = (it >> 1) & 1;
-        const int tk = HH_TASK(task); const int h = tk % p.H, f = (tk / p.H) % p.T, b = tk / (p.H * p.T);
+        const int tk = task_index(task, ntasks); const int h = tk % p.H, f = (tk / p.H) % p.T, b = tk / (p.H * p.T);
         const int cs = it & (NCLS - 1);
         uint8_t* base = smem + st * STAGE_BYTES;
         // tiles in the order their previous contents die: K, Q[0], V, Q[1]
@@ -276,7 +251,7 @@ attn_space_tc_kernel(const __grid_constant__ CUtensorMap tm_in, const __grid_con
     for (int task = blockIdx.x; task < ntasks; task += gridDim.x, ++it) {
       const int st = it & 1;
       const uint32_t ph = (it >> 1) & 1;
-      const int tk = HH_TASK(task); const int h = tk % p.H, f = (tk / p.H) % p.T, b = tk / (p.H * p.T);
+      const int tk = task_index(task, ntasks); const int h = tk % p.H, f = (tk / p.H) % p.T, b = tk / (p.H * p.T);
       const int cs = it & (NCLS - 1);
       // this warp's 64 query rows belong to half ww / 2: their CLS-key logits only need that half of Q (and k_cls)
       mbar_wait(&ex->k_full[st], ph);
@@ -285,7 +260,6 @@ attn_space_tc_kernel(const __grid_constant__ CUtensorMap tm_in, const __grid_con
       const uint32_t qs = smem_u32(smem + st * STAGE_BYTES);
       const uint32_t ks = qs + TILE_BYTES, vs = ks + TILE_BYTES;
 
-#ifndef HH_ATTN_NOHELP
       // ---- (1) CLS-key logit of every query row: S_cls = Q . k_cls, as m16n8k16 with k_cls in column 0 of B
       uint32_t kb0[4], kb1[4];
 #pragma unroll
@@ -313,12 +287,10 @@ attn_space_tc_kernel(const __grid_constant__ CUtensorMap tm_in, const __grid_con
           }
         }
       }
-#endif
       __syncwarp();
       if (lane == 0) mbar_arrive(&ex->scls_full[st][ww >> 1]);
       if (ww == 0 && lane == 0) trace_ev(p, 2, it, 1);
       mbar_wait(&ex->v_full[st], ph);   // part (2) reads K and V
-#ifndef HH_ATTN_NOHELP
 
       // ---- (2) CLS query vs this warp's 64 keys: online softmax over 2 blocks of 32 keys, row 0 of the A block live
       uint32_t qa0[4], qa2[4];
@@ -436,7 +408,6 @@ attn_space_tc_kernel(const __grid_constant__ CUtensorMap tm_in, const __grid_con
           }
         }
       }
-#endif
       asm volatile("bar.sync 2, 128;" ::: "memory");  // merge[] reusable; all four warps are done with Q, K and V
       if (ww == 0 && lane == 0) {
         mbar_arrive(&ex->k_empty[st]);
@@ -468,7 +439,7 @@ attn_space_tc_kernel(const __grid_constant__ CUtensorMap tm_in, const __grid_con
       const int st = u & 1;
       const uint32_t ph = (u >> 1) & 1;
       const uint32_t tp = u & 1;
-      const int tk = HH_TASK(task); const int h = tk % p.H, f = (tk / p.H) % p.T, b = tk / (p.H * p.T);
+      const int tk = task_index(task, ntasks); const int h = tk % p.H, f = (tk / p.H) % p.T, b = tk / (p.H * p.T);
       const uint32_t qs = smem_u32(smem + st * STAGE_BYTES);
       mbar_wait(&ex->scls_full[st][hf], ph);
       const float s_cls = ex->scls[st][r];
@@ -493,17 +464,9 @@ attn_space_tc_kernel(const __grid_constant__ CUtensorMap tm_in, const __grid_con
               if (c * 32 + j < nvalid) mx = fmaxf(mx, __uint_as_float(v[j]));
           }
         };
-#ifdef HH_ATTN_X_NOMAX
-        mq[0] = 8.f;
-        if (false)
-#endif
         tmem_ld_32x32b_x32(s_col, va);
 #pragma unroll 1
-#ifdef HH_ATTN_X_NOMAX
-        for (int c = 0; c < 0; c += 2) {
-#else
         for (int c = 0; c < nch; c += 2) {
-#endif
           tmem_ld_wait();
           if (c + 1 < nch) tmem_ld_32x32b_x32(s_col + (c + 1) * 32, vb);
           fold(va, c);
@@ -522,7 +485,6 @@ attn_space_tc_kernel(const __grid_constant__ CUtensorMap tm_in, const __grid_con
       }
       const float ml = mx * LOG2E;
       const float p_cls = fast_exp2(fmaf(s_cls, LOG2E, -ml));
-#ifndef HH_ATTN_NO_TURNS
       // The exp pass is the one phase that saturates a shared unit (MUFU: 4 lanes per clock and scheduler).  The two warps
       // of a scheduler (same TMEM lane quarter, one per half) take strict turns in it -- h0(u), h1(u), h0(u + 1), ... -- so
       // one half's exponentials always run under the other half's MUFU-free phases (P V wait, read-out, next S, row
@@ -530,7 +492,6 @@ attn_space_tc_kernel(const __grid_constant__ CUtensorMap tm_in, const __grid_con
       // they drift into phase, share the MUFU during the exp pass and leave it idle for the rest of the period.
       if (hf == 1) mbar_wait(&ex->x_done[0][wq], tp);
       else if (u > 0) mbar_wait(&ex->x_done[1][wq], tp ^ 1u);
-#endif
       if (tr) trace_ev(p, 3 + jh, u, 5);
 
       // ---- pass 2: P = exp2(S - max) as bf16 pairs, 32 keys per iteration of ONE small loop body (next to the helper
@@ -539,7 +500,7 @@ attn_space_tc_kernel(const __grid_constant__ CUtensorMap tm_in, const __grid_con
       // first issues the load of the next chunk into x[] (dead), runs this chunk's exponentials on t[], and scales x[] into
       // t[] at the bottom.  (A load whose consumer sits in the next iteration is sunk behind the last reader of its
       // registers, i.e. to the end of the body, and its whole latency is exposed in every chunk.)
-      float2 l2 = make_float2(0.f, 0.f), l2b = make_float2(0.f, 0.f);
+      float2 l2 = make_float2(0.f, 0.f);
       {
         const float2 sc = make_float2(LOG2E, LOG2E), sh = make_float2(-ml, -ml);
         uint32_t x[32];
@@ -558,15 +519,12 @@ attn_space_tc_kernel(const __grid_constant__ CUtensorMap tm_in, const __grid_con
           if (kFull || c < nch) {
 #pragma unroll
             for (int j = 0; j < 16; ++j) {
-              float2 e;
-              if ((j & 3) < HH_ATTN_EMU) e = poly_exp2x2(t[j]);
-              else e = make_float2(fast_exp2(t[j].x), fast_exp2(t[j].y));
+              float2 e = make_float2(fast_exp2(t[j].x), fast_exp2(t[j].y));
               if (!kFull) {   // ragged last chunk (n = 196)
                 if (c * 32 + 2 * j >= nvalid) e.x = 0.f;
                 if (c * 32 + 2 * j + 1 >= nvalid) e.y = 0.f;
               }
-              if ((j & 3) < HH_ATTN_EMU) l2b = __fadd2_rn(l2b, e);
-              else l2 = __fadd2_rn(l2, e);
+              l2 = __fadd2_rn(l2, e);
               w[j] = pack_bf16x2(e.x, e.y);
             }
           } else {
@@ -587,10 +545,8 @@ attn_space_tc_kernel(const __grid_constant__ CUtensorMap tm_in, const __grid_con
           }
         }
       }
-      const float l = (l2.x + l2.y) + (l2b.x + l2b.y) + p_cls;
-#ifndef HH_ATTN_NO_TURNS
+      const float l = (l2.x + l2.y) + p_cls;
       if (lane == 0) mbar_arrive(&ex->x_done[hf][wq]);
-#endif
       if (tr) trace_ev(p, 3 + jh, u, 6);
       {   // the CLS key's probability as key 0 of a 17th K = 16 block (columns [192, 200)); its B tile holds v_cls in row 0
         uint32_t wc[8] = {pack_bf16x2(p_cls, 0.f), 0u, 0u, 0u, 0u, 0u, 0u, 0u};
@@ -631,10 +587,8 @@ attn_space_tc_kernel(const __grid_constant__ CUtensorMap tm_in, const __grid_con
           st_shared_v4(sw128(stg, lane, half32 * 4 + c), wv[0], wv[1], wv[2], wv[3]);
         }
       };
-#ifndef HH_ATTN_X_NOSTAGE
       stage(va, 0);
       stage(vb, 1);
-#endif
       fence_proxy_async_smem();
       __syncwarp();
       if (lane == 0) {
@@ -701,10 +655,7 @@ int make_map4d(CUtensorMap* map, const bf16* base_row1, int cols, int n, int T, 
 
 }  // namespace
 
-bool attn_space_tc_supported(int n) {
-  static const bool off = std::getenv("HH_ATTN_SPACE_MMA_SYNC") != nullptr;
-  return !off && n <= ROWS;
-}
+bool attn_space_tc_supported(int n) { return n <= ROWS; }
 
 int attn_space_tc(const bf16* qkv, bf16* out, int B, int T, int n, int H, float* cls_ws, cudaStream_t stream) {
   HH_REQUIRE(B > 0 && T > 0 && n > 0 && n <= ROWS && H > 0, "attn_space_tc: needs 1 <= n <= 256");

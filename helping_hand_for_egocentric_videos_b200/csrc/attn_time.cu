@@ -1,18 +1,10 @@
 // Temporal half of the divided space-time attention (VarAttention with einops '(b n) f d', model/LaviLa.py:246-283)
 // and the CLS query row shared by both halves.
 //
-// attn_time (T <= 16): patch query (f,p) attends {CLS key} U {(f',p) : f'} -- T+1 <= 17 keys of 64 dims, 16 queries.
-//   HBM-bound (q,k,v read once, o written once).  One warp owns one head of one clip and walks a chunk of patch
-//   positions; per position it pulls the 3*T row segments (128 B each) into its private shared-memory tile with
-//   16-byte cp.async, then runs the 16x24x64 and 16x64x32 products on the legacy tensor-core path (mma.sync
-//   m16n8k16, fp32 accumulate) with an fp32 softmax in registers.  The 8 warps of a CTA cover 8 adjacent heads, so
-//   every global row access of the CTA is a 1 KB contiguous span.
-//   The CLS *query* (which attends all 1+T*n keys, LaviLa.py:258) rides along as a second 16-row MMA block whose
-//   only live row is q_cls: each warp keeps a running (max, sum, o[64]) over the keys it sees and writes ONE partial
-//   per (clip, head, patch-chunk); attn_cls_merge folds the partials and the CLS key itself into output row 0.
+// attn_time (T <= 16) runs the tensor-core kernel of attn_time_v2.cu, which writes one partial of the CLS *query*
+// (which attends all 1+T*n keys, LaviLa.py:258) per (clip, head, patch-chunk); attn_cls_merge folds the partials and the
+// CLS key itself into output row 0.
 // attn_time (16 < T <= 32) keeps the simple SIMT kernel + the stand-alone CLS kernel.
-#include <cstdlib>
-
 #include "hh_internal.h"
 #include "hh_ptx.cuh"
 
@@ -26,205 +18,6 @@ constexpr float LOG2E = 1.4426950408889634f;
 __device__ __forceinline__ void unpack8(const uint4& u, float* f) {
   float2 a = unpack_bf16x2(u.x), b = unpack_bf16x2(u.y), c = unpack_bf16x2(u.z), d = unpack_bf16x2(u.w);
   f[0] = a.x; f[1] = a.y; f[2] = b.x; f[3] = b.y; f[4] = c.x; f[5] = c.y; f[6] = d.x; f[7] = d.y;
-}
-
-// ============================================================================================ tensor-core kernel
-constexpr int TW = 8;            // warps (= adjacent heads) per CTA
-constexpr int TLD = 72;          // smem row stride in bf16 (144 B): conflict-free ldmatrix
-constexpr int TQ_ROWS = 32;      // rows 0..15 queries of the patch problems, row 16 = q_cls, 17..31 zero
-constexpr int TK_ROWS = 24;      // key slots: 0 = CLS, 1..T frames, rest zero
-constexpr int TV_ROWS = 32;      // value slots (second k16 step reads rows 16..31)
-constexpr int TWARP_ELEMS = (TQ_ROWS + TK_ROWS + TV_ROWS) * TLD;
-
-__global__ void __launch_bounds__(TW * 32, 2)
-attn_time_mma_kernel(const bf16* __restrict__ qkv, bf16* __restrict__ out, float* __restrict__ cls_part, int T, int n,
-                     int H, int pchunk, int nchunks) {
-  extern __shared__ __align__(16) uint8_t smem_raw[];
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  bf16* Qs = reinterpret_cast<bf16*>(smem_raw) + static_cast<size_t>(warp) * TWARP_ELEMS;
-  bf16* Ks = Qs + TQ_ROWS * TLD;
-  bf16* Vs = Ks + TK_ROWS * TLD;
-
-  const int D = H * HD;
-  const int N = 1 + T * n;
-  const int hgroups = (H + TW - 1) / TW;
-  const int chunk = blockIdx.x % nchunks;
-  const int hg = (blockIdx.x / nchunks) % hgroups;
-  const int b = blockIdx.x / (nchunks * hgroups);
-  const int h = hg * TW + warp;
-  if (h >= H) return;  // whole warp; no block-level barriers below
-  const size_t ld = static_cast<size_t>(3) * D;
-  const bf16* clip = qkv + static_cast<size_t>(b) * N * ld + h * HD;
-
-  // ---- zero the private tile once (padding rows must stay finite), then the per-warp constants: CLS k, v, q
-  for (int i = lane; i < TWARP_ELEMS / 8; i += 32) reinterpret_cast<uint4*>(Qs)[i] = make_uint4(0, 0, 0, 0);
-  __syncwarp();
-  if (lane < 24) {
-    const int which = lane >> 3, ch = lane & 7;  // 0: q_cls -> Qs row 16, 1: k_cls -> Ks row 0, 2: v_cls -> Vs row 0
-    bf16* dst = (which == 0 ? Qs + 16 * TLD : which == 1 ? Ks : Vs) + ch * 8;
-    cp_async_16(dst, clip + which * D + ch * 8, true);
-  }
-  cp_async_commit();
-
-  const int g = lane >> 2, t = lane & 3;
-  const int mi = lane >> 3, lr = lane & 7;
-  const int nkeys = T + 1;
-
-  // running softmax state of the CLS query over the keys this warp visits (rows g of the second MMA block;
-  // only g == 0 is meaningful)
-  float cm = -INFINITY, cl = 0.f;
-  float co[8][4];
-#pragma unroll
-  for (int ni = 0; ni < 8; ++ni) co[ni][0] = co[ni][1] = co[ni][2] = co[ni][3] = 0.f;
-
-  const int p_begin = chunk * pchunk;
-  const int p_end = min(n, p_begin + pchunk);
-  for (int p = p_begin; p < p_end; ++p) {
-    // ---- stage q (rows 0..T-1), k, v (slots 1..T) of patch position p: 3*T rows x 8 chunks of 16 bytes
-    for (int c = lane; c < 3 * T * 8; c += 32) {
-      const int ch = c & 7;
-      const int r = c >> 3;
-      const int which = r / T, f = r - which * T;
-      const bf16* src = clip + (1 + static_cast<size_t>(f) * n + p) * ld + which * D + ch * 8;
-      bf16* dst = (which == 0 ? Qs + f * TLD : which == 1 ? Ks + (1 + f) * TLD : Vs + (1 + f) * TLD) + ch * 8;
-      cp_async_16(dst, src, true);
-    }
-    cp_async_commit();
-    cp_async_wait<0>();
-    __syncwarp();
-
-    // ---- S = Q K^T for both 16-row blocks (block 1: only row 16 = q_cls is live)
-    float s[2][3][4];
-#pragma unroll
-    for (int mb = 0; mb < 2; ++mb)
-#pragma unroll
-      for (int ni = 0; ni < 3; ++ni) s[mb][ni][0] = s[mb][ni][1] = s[mb][ni][2] = s[mb][ni][3] = 0.f;
-#pragma unroll
-    for (int ks = 0; ks < 4; ++ks) {
-      uint32_t k01[4], k2[4];
-      ldmatrix_x4(k01, smem_u32(Ks + ((mi >> 1) * 8 + lr) * TLD + ks * 16 + (mi & 1) * 8));
-      ldmatrix_x4(k2, smem_u32(Ks + (16 + lr) * TLD + ks * 16 + (mi & 1) * 8));  // matrices 2,3 repeat 0,1 (unused)
-#pragma unroll
-      for (int mb = 0; mb < 2; ++mb) {
-        uint32_t qf[4];
-        ldmatrix_x4(qf, smem_u32(Qs + (mb * 16 + (mi & 1) * 8 + lr) * TLD + ks * 16 + (mi >> 1) * 8));
-        mma_bf16_16816(s[mb][0], qf, k01[0], k01[1]);
-        mma_bf16_16816(s[mb][1], qf, k01[2], k01[3]);
-        mma_bf16_16816(s[mb][2], qf, k2[0], k2[1]);
-      }
-    }
-
-    // ---- patch queries: softmax over the nkeys valid slots, O = P V
-    float mx0 = -INFINITY, mx1 = -INFINITY;
-#pragma unroll
-    for (int ni = 0; ni < 3; ++ni) {
-      const int key = ni * 8 + 2 * t;
-      if (key >= nkeys) s[0][ni][0] = s[0][ni][2] = -INFINITY;
-      if (key + 1 >= nkeys) s[0][ni][1] = s[0][ni][3] = -INFINITY;
-      mx0 = fmaxf(mx0, fmaxf(s[0][ni][0], s[0][ni][1]));
-      mx1 = fmaxf(mx1, fmaxf(s[0][ni][2], s[0][ni][3]));
-    }
-    mx0 = fmaxf(mx0, __shfl_xor_sync(0xffffffffu, mx0, 1));
-    mx0 = fmaxf(mx0, __shfl_xor_sync(0xffffffffu, mx0, 2));
-    mx1 = fmaxf(mx1, __shfl_xor_sync(0xffffffffu, mx1, 1));
-    mx1 = fmaxf(mx1, __shfl_xor_sync(0xffffffffu, mx1, 2));
-    float l0 = 0.f, l1 = 0.f;
-    uint32_t pa[2][4];
-#pragma unroll
-    for (int ni = 0; ni < 3; ++ni) {
-      const float p0 = fast_exp2(fmaf(s[0][ni][0], LOG2E, -mx0 * LOG2E)), p1 = fast_exp2(fmaf(s[0][ni][1], LOG2E, -mx0 * LOG2E));
-      const float p2 = fast_exp2(fmaf(s[0][ni][2], LOG2E, -mx1 * LOG2E)), p3 = fast_exp2(fmaf(s[0][ni][3], LOG2E, -mx1 * LOG2E));
-      l0 += p0 + p1;
-      l1 += p2 + p3;
-      pa[ni >> 1][(ni & 1) * 2 + 0] = pack_bf16x2(p0, p1);
-      pa[ni >> 1][(ni & 1) * 2 + 1] = pack_bf16x2(p2, p3);
-    }
-    pa[1][2] = pa[1][3] = 0u;
-    l0 += __shfl_xor_sync(0xffffffffu, l0, 1);
-    l0 += __shfl_xor_sync(0xffffffffu, l0, 2);
-    l1 += __shfl_xor_sync(0xffffffffu, l1, 1);
-    l1 += __shfl_xor_sync(0xffffffffu, l1, 2);
-
-    // ---- CLS query (row g of block 1): keys 1..T of this position join its running softmax; key 0 (the CLS key
-    //      itself) is added once, by the merge kernel
-    float cmx = -INFINITY;
-#pragma unroll
-    for (int ni = 0; ni < 3; ++ni) {
-      const int key = ni * 8 + 2 * t;
-      if (key >= nkeys || key == 0) s[1][ni][0] = -INFINITY;
-      if (key + 1 >= nkeys) s[1][ni][1] = -INFINITY;
-      cmx = fmaxf(cmx, fmaxf(s[1][ni][0], s[1][ni][1]));
-    }
-    cmx = fmaxf(cmx, __shfl_xor_sync(0xffffffffu, cmx, 1));
-    cmx = fmaxf(cmx, __shfl_xor_sync(0xffffffffu, cmx, 2));
-    const float cmn = fmaxf(cm, cmx);  // finite: T >= 1 gives at least one valid key
-    const float ccorr = fast_exp2((cm - cmn) * LOG2E);
-    cm = cmn;
-    cl *= ccorr;
-    uint32_t pc[2][4];
-#pragma unroll
-    for (int ni = 0; ni < 3; ++ni) {
-      const float p0 = fast_exp2(fmaf(s[1][ni][0], LOG2E, -cmn * LOG2E)), p1 = fast_exp2(fmaf(s[1][ni][1], LOG2E, -cmn * LOG2E));
-      cl += p0 + p1;
-      pc[ni >> 1][(ni & 1) * 2 + 0] = pack_bf16x2(p0, p1);
-      pc[ni >> 1][(ni & 1) * 2 + 1] = 0u;  // rows g+8 of block 1 are dead
-    }
-    pc[1][2] = pc[1][3] = 0u;
-#pragma unroll
-    for (int ni = 0; ni < 8; ++ni) {
-      co[ni][0] *= ccorr;
-      co[ni][1] *= ccorr;
-    }
-
-    float o[8][4];
-#pragma unroll
-    for (int ni = 0; ni < 8; ++ni) o[ni][0] = o[ni][1] = o[ni][2] = o[ni][3] = 0.f;
-#pragma unroll
-    for (int kk = 0; kk < 2; ++kk) {
-#pragma unroll
-      for (int dp = 0; dp < 4; ++dp) {
-        uint32_t vf[4];
-        ldmatrix_x4_trans(vf, smem_u32(Vs + (kk * 16 + (mi & 1) * 8 + lr) * TLD + dp * 16 + (mi >> 1) * 8));
-        mma_bf16_16816(o[2 * dp], pa[kk], vf[0], vf[1]);
-        mma_bf16_16816(o[2 * dp + 1], pa[kk], vf[2], vf[3]);
-        mma_bf16_16816(co[2 * dp], pc[kk], vf[0], vf[1]);
-        mma_bf16_16816(co[2 * dp + 1], pc[kk], vf[2], vf[3]);
-      }
-    }
-
-    // ---- stage the 16x64 result over the (consumed) query rows, then 16-byte coalesced row stores
-    const float i0 = 1.f / l0, i1 = 1.f / l1;
-    __syncwarp();
-#pragma unroll
-    for (int ni = 0; ni < 8; ++ni) {
-      *reinterpret_cast<uint32_t*>(Qs + g * TLD + ni * 8 + 2 * t) = pack_bf16x2(o[ni][0] * i0, o[ni][1] * i0);
-      *reinterpret_cast<uint32_t*>(Qs + (g + 8) * TLD + ni * 8 + 2 * t) = pack_bf16x2(o[ni][2] * i1, o[ni][3] * i1);
-    }
-    __syncwarp();
-    for (int c = lane; c < T * 8; c += 32) {
-      const int f = c >> 3, ch = c & 7;
-      const uint4 v = *reinterpret_cast<const uint4*>(Qs + f * TLD + ch * 8);
-      bf16* dst = out + (static_cast<size_t>(b) * N + 1 + static_cast<size_t>(f) * n + p) * D + h * HD + ch * 8;
-      *reinterpret_cast<uint4*>(dst) = v;
-    }
-    __syncwarp();  // Qs rows are rewritten by the next position's loads
-  }
-
-  // ---- this warp's CLS partial: (m, l, o[64]) for (b, h, chunk); row 0 of block 1 lives in lanes 0..3
-  cl += __shfl_xor_sync(0xffffffffu, cl, 1);
-  cl += __shfl_xor_sync(0xffffffffu, cl, 2);
-  if (g == 0) {
-    float* dst = cls_part + ((static_cast<size_t>(b) * H + h) * nchunks + chunk) * (HD + 2);
-    if (t == 0) {
-      dst[0] = cm;
-      dst[1] = cl;
-    }
-#pragma unroll
-    for (int ni = 0; ni < 8; ++ni) {
-      dst[2 + ni * 8 + 2 * t] = co[ni][0];
-      dst[2 + ni * 8 + 2 * t + 1] = co[ni][1];
-    }
-  }
 }
 
 // Folds the per-chunk partials of the CLS query and the CLS key/value itself into output row 0 of every (clip, head).
@@ -475,24 +268,8 @@ int attn_time(const bf16* qkv, bf16* out, int B, int T, int n, int H, float* cls
     HH_REQUIRE(cls_ws != nullptr, "attn_time: CLS workspace");
     const int pchunk = 16;
     const int nchunks = (n + pchunk - 1) / pchunk;
-    static const bool use_v1 = std::getenv("HH_ATTN_TIME_V1") != nullptr;
-    if (!use_v1) {  // double-buffered, swizzled-tile generation of the same kernel (attn_time_v2.cu)
-      int rc = attn_time_v2(qkv, out, B, T, n, H, cls_ws, pchunk, nchunks, stream);
-      if (rc) return rc;
-      return attn_cls_merge(qkv, cls_ws, out, B, 1 + T * n, H, nchunks, stream);
-    }
-    const size_t smem = static_cast<size_t>(TW) * TWARP_ELEMS * sizeof(bf16);
-    static bool configured = false;
-    if (!configured) {
-      HH_CHECK_CUDA(cudaFuncSetAttribute(attn_time_mma_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                         static_cast<int>(smem)));
-      configured = true;
-    }
-    const long long blocks = static_cast<long long>(B) * ((H + TW - 1) / TW) * nchunks;
-    HH_REQUIRE(blocks < (1ll << 31), "attn_time: grid too large");
-    attn_time_mma_kernel<<<static_cast<unsigned>(blocks), TW * 32, smem, stream>>>(qkv, out, cls_ws, T, n, H, pchunk,
-                                                                                   nchunks);
-    HH_CHECK_LAUNCH("attn_time_mma_kernel");
+    int rc = attn_time_v2(qkv, out, B, T, n, H, cls_ws, pchunk, nchunks, stream);
+    if (rc) return rc;
     return attn_cls_merge(qkv, cls_ws, out, B, 1 + T * n, H, nchunks, stream);
   }
   int rc = launch_time<32>(qkv, out, B, T, n, H, stream);

@@ -1,4 +1,10 @@
-// Temporal attention, second generation of the mma.sync kernel in attn_time.cu (same math, same CLS-query partials):
+// Temporal attention for T <= 16 (attn_time in attn_time.cu): patch query (f,p) attends {CLS key} U {(f',p) : f'} --
+// T+1 <= 17 keys of 64 dims, 16 queries.  HBM-bound (q,k,v read once, o written once).  One warp owns one head of one clip
+// and walks a chunk of patch positions; per position it runs the 16x24x64 and 16x64x32 products on the legacy
+// tensor-core path (mma.sync m16n8k16, fp32 accumulate) with an fp32 softmax in registers.  The 8 warps of a CTA cover 8
+// adjacent heads, so every global row access of the CTA is a 1 KB contiguous span.  The CLS *query* rides along as a
+// second 16-row MMA block whose only live row is q_cls: each warp keeps a running (max, sum, o[64]) over the keys it sees
+// and writes ONE partial per (clip, head, patch-chunk) for attn_cls_merge.
 //   * per-warp shared-memory tiles are 128-byte rows with an XOR swizzle instead of padded rows, and the key / value /
 //     query slots that are constant (CLS row) or always zero are single shared rows addressed per lane by ldmatrix,
 //     so a warp needs 12.5 KB and its loads can be DOUBLE-BUFFERED: the 3*T row segments of patch position p+1 are in
@@ -6,8 +12,8 @@
 //   * the frame count is a template parameter for T = 4 / 8 / 16 (every configuration the reference runs): the copy
 //     loops are fully unrolled over per-lane base pointers + warp-uniform offsets, so a 16-byte cp.async costs ~2
 //     instructions instead of the ~60 of the runtime-T index arithmetic (integer division by T, swizzle, 64-bit
-//     address) that made the first version issue-bound at 46 % of HBM bandwidth. TT = 0 keeps the runtime-T loops.
-#include <cstdlib>
+//     address) that made the first version issue-bound at 46 % of HBM bandwidth. TT = 0 runs the runtime-T loops for
+//     every other T.
 #include "hh_internal.h"
 #include "hh_ptx.cuh"
 
@@ -45,11 +51,7 @@ attn_time_v2_kernel(const bf16* __restrict__ qkv, bf16* __restrict__ out, float*
   const int chunk = blockIdx.x % nchunks;
   const int hg = (blockIdx.x / nchunks) % hgroups;
   // last clips first: their q/k/v rows were written last by the QKV GEMM and are still in L2 (see rows.cu)
-#ifdef HH_FORWARD_WALK
-  const int b = blockIdx.x / (nchunks * hgroups);
-#else
   const int b = static_cast<int>(gridDim.x) / (nchunks * hgroups) - 1 - static_cast<int>(blockIdx.x) / (nchunks * hgroups);
-#endif
   const int h = hg * TW + warp;
   if (h >= H) return;  // whole warp; no block-level barriers below
   const size_t ld = static_cast<size_t>(3) * D;
@@ -313,12 +315,9 @@ static int launch_v2(const bf16* qkv, bf16* out, int B, int T, int n, int H, flo
 
 int attn_time_v2(const bf16* qkv, bf16* out, int B, int T, int n, int H, float* cls_ws, int pchunk, int nchunks,
                  cudaStream_t stream) {
-  static const bool generic = std::getenv("HH_ATTN_TIME_GENERIC") != nullptr;  // differential testing of the TT paths
-  if (!generic) {
-    if (T == 16) return launch_v2<16>(qkv, out, B, T, n, H, cls_ws, pchunk, nchunks, stream);
-    if (T == 8) return launch_v2<8>(qkv, out, B, T, n, H, cls_ws, pchunk, nchunks, stream);
-    if (T == 4) return launch_v2<4>(qkv, out, B, T, n, H, cls_ws, pchunk, nchunks, stream);
-  }
+  if (T == 16) return launch_v2<16>(qkv, out, B, T, n, H, cls_ws, pchunk, nchunks, stream);
+  if (T == 8) return launch_v2<8>(qkv, out, B, T, n, H, cls_ws, pchunk, nchunks, stream);
+  if (T == 4) return launch_v2<4>(qkv, out, B, T, n, H, cls_ws, pchunk, nchunks, stream);
   return launch_v2<0>(qkv, out, B, T, n, H, cls_ws, pchunk, nchunks, stream);
 }
 

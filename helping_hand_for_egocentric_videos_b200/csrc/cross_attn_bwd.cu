@@ -14,9 +14,8 @@
 // lse comes from the forward (cross_attn's lse_out) or is recomputed by cross_stats_kernel; D_i = dO_i . O_i is taken
 // per CTA.  Every warp leaves a partial dq [16 x 64]; cross_dq_merge_kernel adds the partials in a fixed order (no
 // atomics: dq is bit-reproducible).  The first-generation SIMT statement (decoder_bwd.cu: one thread per key, dS through
-// HBM, 5 ms per c4 backward) stays behind HH_CROSS_BWD_SIMT=1 as the differential reference.
-#include <cstdlib>
-
+// HBM, 5 ms per c4 backward) serves the inputs this kernel does not take: q / dO that are not 8-byte aligned, dK / dV that
+// are not 4-byte aligned, and dropout with a key count that is not a multiple of 8.
 #include "hh_internal.h"
 #include "hh_ptx.cuh"
 
@@ -282,14 +281,6 @@ int bwd_splits(int B, int heads, int S) {
   return splits;
 }
 
-bool simt_forced() {
-  static const bool on = [] {
-    const char* e = std::getenv("HH_CROSS_BWD_SIMT");
-    return e && e[0] == '1';
-  }();
-  return on;
-}
-
 }  // namespace
 
 size_t cross_attn_bwd_workspace_bytes(int B, int Q, int heads, int S) {
@@ -308,7 +299,7 @@ int cross_attn_bwd(const float* q, const bf16* K, const bf16* V, int ldkv, const
   const bool aligned = (reinterpret_cast<uintptr_t>(K) & 15) == 0 && (reinterpret_cast<uintptr_t>(V) & 15) == 0 &&
                        (reinterpret_cast<uintptr_t>(q) & 7) == 0 && (reinterpret_cast<uintptr_t>(dO) & 7) == 0 &&
                        (reinterpret_cast<uintptr_t>(dK) & 3) == 0 && (reinterpret_cast<uintptr_t>(dV) & 3) == 0;
-  if (simt_forced() || !aligned || (drop.thr != 0 && S % 8 != 0))
+  if (!aligned || (drop.thr != 0 && S % 8 != 0))
     return cross_attn_bwd_simt(q, K, V, ldkv, O, dO, dq, dK, dV, lddkv, B, Q, heads, S, workspace, s, drop, drop_site, lse_saved);
   float* lse_ws = static_cast<float*>(workspace);
   float* part = lse_ws + static_cast<size_t>(B) * heads * Q;

@@ -12,7 +12,6 @@
 // The class head has no loss in the reference's criterion (losses = ['boxes', 'cardinality'], run/train.py:471;
 // exclude_class=True), so class_embed receives zero gradients.  Host-side C++ only (kernels: decoder_bwd.cu).
 #include <cmath>
-#include <cstdlib>
 
 #include "engine.h"
 
@@ -165,27 +164,21 @@ int Decoder::backward(const float* hs, const float* boxes, const float* d_hs, co
   // ---- The weight gradients run on a second stream beside the data-gradient chain: at the query side's sizes neither
   // fills the GPU (208-CTA launches, latency-bound).  fork() orders a weight gradient after everything issued so far;
   // side_reads(slot) marks the scratch buffer it still reads, before_write(slot) makes the main stream wait for that
-  // reader before a later kernel overwrites the buffer.  HH_BWD_SINGLE_STREAM=1 puts everything back on one stream.
-  static const bool single_stream = [] {
-    const char* e = std::getenv("HH_BWD_SINGLE_STREAM");
-    return e && e[0] == '1';
-  }();
+  // reader before a later kernel overwrites the buffer.
   enum { SL_DX = 0, SL_GA, SL_GB, SL_TMP2, SL_DQKV, SL_N };
-  if (!single_stream && bw_side == nullptr) {
+  if (bw_side == nullptr) {
     HH_CHECK_CUDA(cudaStreamCreateWithFlags(&bw_side, cudaStreamNonBlocking));
     HH_CHECK_CUDA(cudaEventCreateWithFlags(&bw_fork, cudaEventDisableTiming));
     for (int i = 0; i < SL_N; ++i) HH_CHECK_CUDA(cudaEventCreateWithFlags(&bw_done[i], cudaEventDisableTiming));
   }
-  cudaStream_t sw = single_stream ? s : bw_side;
+  cudaStream_t sw = bw_side;
   bool pending[SL_N] = {false, false, false, false, false};
   auto fork = [&]() -> int {
-    if (single_stream) return 0;
     HH_CHECK_CUDA(cudaEventRecord(bw_fork, s));
     HH_CHECK_CUDA(cudaStreamWaitEvent(sw, bw_fork, 0));
     return 0;
   };
   auto side_reads = [&](int slot) -> int {
-    if (single_stream) return 0;
     HH_CHECK_CUDA(cudaEventRecord(bw_done[slot], sw));
     pending[slot] = true;
     return 0;
@@ -337,10 +330,8 @@ int Decoder::backward(const float* hs, const float* boxes, const float* d_hs, co
     RC(ln_bwd(A.x0, p + "norm1", tmp, 0.f));
   }
   // join: the memory side reuses ga / gb, and the caller reads the gradients in stream order
-  if (!single_stream) {
-    HH_CHECK_CUDA(cudaEventRecord(bw_fork, sw));
-    HH_CHECK_CUDA(cudaStreamWaitEvent(s, bw_fork, 0));
-  }
+  HH_CHECK_CUDA(cudaEventRecord(bw_fork, sw));
+  HH_CHECK_CUDA(cudaStreamWaitEvent(s, bw_fork, 0));
   // dx now holds the gradient w.r.t. the zero-initialised tgt: no parameter behind it
 
   // =========================================================================================== memory side

@@ -16,7 +16,6 @@
 #include "hh_internal.h"
 #include "hh_ptx.cuh"
 
-#include <cstdlib>
 #include <mutex>
 #include <unordered_map>
 
@@ -28,14 +27,10 @@ constexpr int BLOCK_M = 128;
 constexpr int BLOCK_K = 64;   // 64 bf16 = one 128-byte swizzle row
 constexpr int UMMA_K = 16;
 constexpr int NUM_THREADS = 256;
-// Warp roles.  HH_GEMM_ROLES_HI (default): the epilogue takes warps 0..3 and the single-thread roles the HIGHEST warp ids --
-// the SMSP arbiter prefers the highest eligible warp id (B300_MICROARCH.md), so the TMA producer and the MMA issuer are
-// never kept waiting by the epilogue warp that shares their scheduler, however instruction-heavy the epilogue is.
-#ifndef HH_GEMM_ROLES_LO
+// Warp roles: the epilogue takes warps 0..3 and the single-thread roles the HIGHEST warp ids -- the SMSP arbiter prefers
+// the highest eligible warp id (B300_MICROARCH.md), so the TMA producer and the MMA issuer are never kept waiting by the
+// epilogue warp that shares their scheduler, however instruction-heavy the epilogue is.
 constexpr int EPI_WARP0 = 0, W_ALLOC = 4, W_RES = 5, W_PROD = 6, W_MMA = 7;
-#else   // round-1 numbering (A/B)
-constexpr int EPI_WARP0 = 4, W_ALLOC = 2, W_RES = 3, W_PROD = 0, W_MMA = 1;
-#endif
 constexpr int STAGE_LD = 33;  // per-warp transpose buffer: 32 rows x 33 words
 
 // DEEP_EPI (the QuickGELU epilogue of the 2-SM path): a 4-slot store ring per epilogue warp and one operand stage fewer
@@ -43,22 +38,16 @@ constexpr int STAGE_LD = 33;  // per-warp transpose buffer: 32 rows x 33 words
 // operand stage (qkv 61.7 -> 62.6 ms with the deep ring), so they keep 2 slots.
 // RES (the residual + LayerNorm-statistics epilogue): a per-warp ring of RES_SLOTS fp32 boxes (32 rows x 32 columns, 4 KB)
 // that the residual tile streams through (TMA load -> add in place -> TMA store), paid for with two operand stages.
-// LONGK (the K >= 2048 residual producer, fc2): its epilogue idles ~70 % of a tile, so it gives one z slot and one residual
-// slot back to the operand ring (5 stages instead of 4: the plain fc2 loses 5.5 % with 4 stages instead of 6).
-template <int BLOCK_N, bool TWOSM = false, bool DEEP_EPI = false, bool RES = false, bool LNF = false, bool LONGK = false>
+// It runs on 2-SM 256-wide and unclustered 128-wide tiles only (plan_tiles).
+template <int BLOCK_N, bool TWOSM = false, bool DEEP_EPI = false, bool RES = false, bool LNF = false>
 struct Cfg {
   static constexpr int A_BYTES = BLOCK_M * BLOCK_K * 2;
   static constexpr int B_BYTES = (TWOSM ? BLOCK_N / 2 : BLOCK_N) * BLOCK_K * 2;  // per CTA
   static constexpr int STAGE_BYTES = A_BYTES + B_BYTES;
-  static constexpr int RES_SLOTS = LONGK ? 3 : 4;
+  static constexpr int RES_SLOTS = 4;
   static constexpr int RES_BYTES = RES ? 4 * RES_SLOTS * 4096 : 0;
-#ifdef HH_GEMM_PLAIN_STAGES   // variant builds: sensitivity of the plain epilogues to the operand ring depth
-  static constexpr int STAGES = RES ? ((BLOCK_N == 256 && !TWOSM) ? 2 : (LONGK ? 5 : 4)) : ((BLOCK_N == 256 && !TWOSM) ? 4 : HH_GEMM_PLAIN_STAGES);
-#else
-  static constexpr int STAGES = RES ? ((BLOCK_N == 256 && !TWOSM) ? 2 : (LONGK ? 5 : 4))
-                                    : ((BLOCK_N == 256 && !TWOSM) ? 4 : ((TWOSM && DEEP_EPI) ? 5 : 6));
-#endif
-  static constexpr int EPI_SLOTS = (TWOSM && DEEP_EPI) ? 4 : (LONGK ? 1 : 2);  // per-warp ring of 32-row x 128-byte store slots
+  static constexpr int STAGES = RES ? 4 : ((BLOCK_N == 256 && !TWOSM) ? 4 : ((TWOSM && DEEP_EPI) ? 5 : 6));
+  static constexpr int EPI_SLOTS = (TWOSM && DEEP_EPI) ? 4 : 2;  // per-warp ring of 32-row x 128-byte store slots
   static constexpr int EPI_BYTES = 4 * EPI_SLOTS * 4096;            // (>= the 4 x 32 x 33 words of the direct path)
   static constexpr int BIAS_BYTES = (LNF ? 2 : 1) * BLOCK_N * 4;    // bias tile (+ column-sum tile: LayerNorm-folded GEMMs)
   static constexpr int BAR_BYTES = RES ? 512 : 256;
@@ -142,7 +131,7 @@ __device__ __forceinline__ void st_shared_v4(uint32_t addr, uint32_t a, uint32_t
 // 32 KB instead of 48 KB (6 stages instead of 4).  Barrier protocol: both producers' TMA loads complete on the LEADER's
 // full barrier (which expects both CTAs' bytes); the leader's commits are multicast to both CTAs' empty / accumulator-
 // full barriers; both CTAs' epilogue warps arrive on the LEADER's accumulator-empty barrier.
-template <int BLOCK_N, int EPI, bool TMA_STORE, bool CLUSTER, bool TWOSM = false, bool LONGK = false>
+template <int BLOCK_N, int EPI, bool TMA_STORE, bool CLUSTER, bool TWOSM = false>
 __global__ void __launch_bounds__(NUM_THREADS, 1)
 gemm_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constant__ CUtensorMap tma_b,
             const __grid_constant__ CUtensorMap tma_c, const __grid_constant__ CUtensorMap tma_r, const GemmArgs p) {
@@ -151,8 +140,7 @@ gemm_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constant__ C
   constexpr bool LNF = (EPI == EPI_LN_BIAS_BF16 || EPI == EPI_LN_BIAS_QGELU_BF16);   // LayerNorm folded (consumer side)
   constexpr bool RES = (EPI == EPI_RES_STATS_BF16);                                  // residual + statistics (producer)
   static_assert(!(LNF || RES) || TMA_STORE, "the fused-LayerNorm epilogues use bulk-tensor stores");
-  static_assert(!LONGK || (EPI == EPI_RES_STATS_BF16 && TWOSM), "the long-K plan belongs to the 2-SM residual producer");
-  using C = Cfg<BLOCK_N, TWOSM, QGELU, RES, LNF, LONGK>;
+  using C = Cfg<BLOCK_N, TWOSM, QGELU, RES, LNF>;
   extern __shared__ __align__(1024) uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
   if constexpr (C::ALIGN_SLACK == 0) {
@@ -321,9 +309,6 @@ gemm_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constant__ C
         uint64_t* const my_full = res_full + q * C::RES_SLOTS;
         uint64_t* const my_empty = res_empty + q * C::RES_SLOTS;
         uint8_t* const my_ring = res_stage + q * C::RES_SLOTS * 4096;
-#ifdef HH_GEMM_RES_HINTS
-        const uint64_t res_policy = l2_policy_evict_first();   // the residual is read once per GEMM
-#endif
         int slot = 0;
         uint32_t phase = 0;
         for (int tile = tile_first; tile < total_tiles; tile += tile_step) {
@@ -332,17 +317,9 @@ gemm_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constant__ C
           const int m_blk = CLUSTER ? 2 * mp + cta_rank : mp;
 #pragma unroll 1
           for (int u = 0; u < BLOCK_N / 32; ++u) {
-#ifdef HH_GEMM_RES_NOLOAD   // experiment: the producer epilogue without its residual loads (results are wrong)
-            continue;
-#endif
             mbar_wait(&my_empty[slot], phase ^ 1u);
             mbar_arrive_expect_tx(&my_full[slot], 4096);
-#ifdef HH_GEMM_RES_HINTS
-            tma_load_2d_hint(&tma_r, &my_full[slot], my_ring + slot * 4096, n_blk * BLOCK_N + u * 32, m_blk * BLOCK_M + q * 32,
-                             res_policy);
-#else
             tma_load_2d(&tma_r, &my_full[slot], my_ring + slot * 4096, n_blk * BLOCK_N + u * 32, m_blk * BLOCK_M + q * 32);
-#endif
             if (++slot == C::RES_SLOTS) {
               slot = 0;
               phase ^= 1u;
@@ -452,9 +429,7 @@ gemm_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constant__ C
           const uint32_t slot = static_cast<uint32_t>(res_slot);
           uint32_t r[32];
           tmem_ld_32x32b_x32(t_row + static_cast<uint32_t>(u * 32), r);   // in flight while the residual box is awaited
-#ifndef HH_GEMM_RES_NOLOAD
           { TR_T0(); mbar_wait(&my_res_full[slot], res_phase); TR_ADD(5); }
-#endif
           const uint32_t rrow = res_ring + slot * 4096u + static_cast<uint32_t>(lane * 128);
           const uint32_t zrow = zring + static_cast<uint32_t>(epi_slot * 4096 + lane * 128);
           tmem_ld_wait();
@@ -485,11 +460,7 @@ gemm_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constant__ C
           fence_proxy_async_smem();
           __syncwarp();
           if (lane == 0) {
-#ifdef HH_GEMM_RES_HINTS
-            if (p.writeback) tma_store_2d_hint(&tma_r, res_ring + slot * 4096u, col0 + u * 32, row0, l2_policy_evict_first());
-#else
             if (p.writeback) tma_store_2d(&tma_r, res_ring + slot * 4096u, col0 + u * 32, row0);
-#endif
             if (u & 1) tma_store_2d(&tma_c, zring + static_cast<uint32_t>(epi_slot * 4096), col0 + (u >> 1) * 64, row0);
             tma_store_commit();
             // every group but the newest has been read out of shared memory: with write-back that frees the previous
@@ -540,11 +511,6 @@ gemm_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constant__ C
 #pragma unroll
               for (int j = 0; j < 32; j += 2) {
                 // packed fp32x2 arithmetic (same IEEE results as the scalar ops, half the issue slots / energy)
-#ifdef HH_SCALAR_EPI   // A/B switch: the scalar statement of the same arithmetic
-                float2 v = make_float2(__uint_as_float(r[j]) + bias_s[c * 64 + h * 32 + j],
-                                       __uint_as_float(r[j + 1]) + bias_s[c * 64 + h * 32 + j + 1]);
-                if constexpr (EPI == EPI_BIAS_QGELU_BF16) v = make_float2(quick_gelu(v.x), quick_gelu(v.y));
-#else
                 float2 v;
                 if constexpr (LNF) {  // rstd * acc + (bias' - rstd * mean * colsum)
                   const float2 t = __ffma2_rn(*reinterpret_cast<const float2*>(&cs_s[c * 64 + h * 32 + j]), ln_nm,
@@ -555,7 +521,6 @@ gemm_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constant__ C
                                  *reinterpret_cast<const float2*>(&bias_s[c * 64 + h * 32 + j]));
                 }
                 if constexpr (QGELU) v = quick_gelu2(v);
-#endif
                 w[j >> 1] = pack_bf16x2(v.x, v.y);
               }
 #pragma unroll
@@ -716,13 +681,13 @@ int make_tmap(CUtensorMap* map, const void* base, int rows, int cols, int ld, in
   return 0;
 }
 
-template <int BLOCK_N, int EPI, bool TMA_STORE, bool CLUSTER, bool TWOSM = false, bool LONGK = false>
+template <int BLOCK_N, int EPI, bool TMA_STORE, bool CLUSTER, bool TWOSM = false>
 int launch(const CUtensorMap& ta, const CUtensorMap& tb, const CUtensorMap& tc, const CUtensorMap& tr, const GemmArgs& args,
            cudaStream_t stream) {
   using C = Cfg<BLOCK_N, TWOSM, EPI == EPI_BIAS_QGELU_BF16 || EPI == EPI_LN_BIAS_QGELU_BF16, EPI == EPI_RES_STATS_BF16,
-                EPI == EPI_LN_BIAS_BF16 || EPI == EPI_LN_BIAS_QGELU_BF16, LONGK>;
+                EPI == EPI_LN_BIAS_BF16 || EPI == EPI_LN_BIAS_QGELU_BF16>;
   static bool configured = false;
-  auto kern = gemm_kernel<BLOCK_N, EPI, TMA_STORE, CLUSTER, TWOSM, LONGK>;
+  auto kern = gemm_kernel<BLOCK_N, EPI, TMA_STORE, CLUSTER, TWOSM>;
   if (!configured) {
     HH_CHECK_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, C::SMEM_BYTES));
     configured = true;
@@ -756,25 +721,20 @@ int launch(const CUtensorMap& ta, const CUtensorMap& tb, const CUtensorMap& tc, 
 
 template <int BLOCK_N>
 int dispatch_epi(const CUtensorMap& ta, const CUtensorMap& tb, const CUtensorMap& tc, const CUtensorMap& tr, bool tma_store,
-                 bool cluster, bool twosm, const GemmArgs& args, int epi, cudaStream_t stream) {
-  if constexpr (BLOCK_N == 256) {
-    if (tma_store && cluster && twosm) {
-      switch (epi) {
-        case EPI_BIAS_BF16: return launch<256, EPI_BIAS_BF16, true, true, true>(ta, tb, tc, tr, args, stream);
-        case EPI_BIAS_QGELU_BF16: return launch<256, EPI_BIAS_QGELU_BF16, true, true, true>(ta, tb, tc, tr, args, stream);
-        case EPI_BIAS_F32: return launch<256, EPI_BIAS_F32, true, true, true>(ta, tb, tc, tr, args, stream);
-        case EPI_LN_BIAS_BF16: return launch<256, EPI_LN_BIAS_BF16, true, true, true>(ta, tb, tc, tr, args, stream);
-        case EPI_LN_BIAS_QGELU_BF16:
-          return launch<256, EPI_LN_BIAS_QGELU_BF16, true, true, true>(ta, tb, tc, tr, args, stream);
-        case EPI_RES_STATS_BF16: {
-          // The 5-stage plan cuts the stand-alone fc2 producer from +24 % to +7.6 % over the plain epilogue (cycles), but
-          // inside the power-capped step the launch takes the same time (47.4 vs 47.3 ms per step, A/B on one box):
-          // opt-in until that changes (HH_GEMM_LONGK=1).
-          static const bool longk_ok = std::getenv("HH_GEMM_LONGK") != nullptr;
-          if (longk_ok && args.K >= 2048) return launch<256, EPI_RES_STATS_BF16, true, true, true, true>(ta, tb, tc, tr, args, stream);
-          return launch<256, EPI_RES_STATS_BF16, true, true, true>(ta, tb, tc, tr, args, stream);
-        }
-      }
+                 bool cluster, const GemmArgs& args, int epi, cudaStream_t stream) {
+  // CTA pairs: one 2-SM MMA on 256-wide tiles, two 1-SM MMAs with the W tile multicast on 128-wide tiles
+  constexpr bool TWOSM = BLOCK_N == 256;
+  if (cluster) {
+    switch (epi) {
+      case EPI_BIAS_BF16: return launch<BLOCK_N, EPI_BIAS_BF16, true, true, TWOSM>(ta, tb, tc, tr, args, stream);
+      case EPI_BIAS_QGELU_BF16: return launch<BLOCK_N, EPI_BIAS_QGELU_BF16, true, true, TWOSM>(ta, tb, tc, tr, args, stream);
+      case EPI_BIAS_F32: return launch<BLOCK_N, EPI_BIAS_F32, true, true, TWOSM>(ta, tb, tc, tr, args, stream);
+      case EPI_LN_BIAS_BF16: return launch<BLOCK_N, EPI_LN_BIAS_BF16, true, true, TWOSM>(ta, tb, tc, tr, args, stream);
+      case EPI_LN_BIAS_QGELU_BF16:
+        return launch<BLOCK_N, EPI_LN_BIAS_QGELU_BF16, true, true, TWOSM>(ta, tb, tc, tr, args, stream);
+      case EPI_RES_STATS_BF16:
+        if constexpr (TWOSM) return launch<256, EPI_RES_STATS_BF16, true, true, true>(ta, tb, tc, tr, args, stream);
+        break;
     }
   }
   if (epi == EPI_RES_STATS_BF16) {  // outside the 2-SM path the residual epilogue runs unclustered on 128-wide tiles
@@ -782,15 +742,6 @@ int dispatch_epi(const CUtensorMap& ta, const CUtensorMap& tb, const CUtensorMap
       if (tma_store && !cluster) return launch<128, EPI_RES_STATS_BF16, true, false>(ta, tb, tc, tr, args, stream);
     }
     return fail(-2, "gemm_bf16: residual-statistics epilogue: unsupported tile configuration");
-  }
-  if (tma_store && cluster) {
-    switch (epi) {
-      case EPI_BIAS_BF16: return launch<BLOCK_N, EPI_BIAS_BF16, true, true>(ta, tb, tc, tr, args, stream);
-      case EPI_BIAS_QGELU_BF16: return launch<BLOCK_N, EPI_BIAS_QGELU_BF16, true, true>(ta, tb, tc, tr, args, stream);
-      case EPI_BIAS_F32: return launch<BLOCK_N, EPI_BIAS_F32, true, true>(ta, tb, tc, tr, args, stream);
-      case EPI_LN_BIAS_BF16: return launch<BLOCK_N, EPI_LN_BIAS_BF16, true, true>(ta, tb, tc, tr, args, stream);
-      case EPI_LN_BIAS_QGELU_BF16: return launch<BLOCK_N, EPI_LN_BIAS_QGELU_BF16, true, true>(ta, tb, tc, tr, args, stream);
-    }
   }
   if (tma_store) {
     switch (epi) {
@@ -813,7 +764,7 @@ int dispatch_epi(const CUtensorMap& ta, const CUtensorMap& tb, const CUtensorMap
 // Tile plan shared by the launcher and by callers that size the statistics buffer.
 struct TilePlan {
   int bn, tiles_m, tiles_n;
-  bool cluster, twosm;
+  bool cluster;
 };
 TilePlan plan_tiles(int M, int N, int epilogue, bool tma_store) {
   TilePlan t;
@@ -823,13 +774,11 @@ TilePlan plan_tiles(int M, int N, int epilogue, bool tma_store) {
   if (N <= 128 || (N % 256 != 0 && N % 128 == 0) || t.tiles_m * ((N + 255) / 256) < num_sms()) t.bn = 128;
   // (Measured at the 5-clip EgoMCQ shape, 41 row tiles: choosing 128-wide tiles by wave count loses -- qkv 41.9 vs 31.1 us,
   // proj 22.4 vs 16.7, fc1 52.1 vs 37.3, fc2 59.2 vs 45.4 -- a 128-wide tile costs far more than half a 256-wide one.)
-  // CTA pairs sharing the W tile (multicast) once there are enough row tiles to pair up
-  static const bool cluster_ok = std::getenv("HH_GEMM_NO_CLUSTER") == nullptr;
-  t.cluster = cluster_ok && tma_store && t.tiles_m >= num_sms() / 2 && (num_sms() % 2 == 0);
-  // CTA pairs on one 256-row MMA (cta_group::2) for the wide tiles; HH_GEMM_1SM=1 keeps the multicast 1-SM pairs
-  static const bool twosm_ok = std::getenv("HH_GEMM_1SM") == nullptr;
-  t.twosm = t.cluster && twosm_ok && t.bn == 256;
-  if (epilogue == EPI_RES_STATS_BF16 && !t.twosm) {  // its shared-memory plan exists for 2-SM 256-wide and plain 128-wide tiles
+  // CTA pairs once there are enough row tiles to pair up: one 256-row MMA (cta_group::2) on the wide tiles, the W tile
+  // multicast to two 1-SM MMAs on the 128-wide ones
+  t.cluster = tma_store && t.tiles_m >= num_sms() / 2 && (num_sms() % 2 == 0);
+  // the residual epilogue's shared-memory plan exists for 2-SM 256-wide and plain 128-wide tiles
+  if (epilogue == EPI_RES_STATS_BF16 && !(t.cluster && t.bn == 256)) {
     t.bn = 128;
     t.cluster = false;
   }
@@ -927,8 +876,8 @@ static int gemm_impl(const bf16* A, int lda, int seg_rows, int seg_pitch, const 
   args.writeback = fuse.writeback;
   args.a_seg_rows = seg_rows > 0 ? seg_rows : 0;
   args.a_seg_skip = seg_rows > 0 ? seg_pitch - seg_rows : 0;
-  if (bn == 256) return dispatch_epi<256>(ta, tb, tc, tr, tma_store, t.cluster, t.twosm, args, epilogue, stream);
-  return dispatch_epi<128>(ta, tb, tc, tr, tma_store, t.cluster, false, args, epilogue, stream);
+  if (bn == 256) return dispatch_epi<256>(ta, tb, tc, tr, tma_store, t.cluster, args, epilogue, stream);
+  return dispatch_epi<128>(ta, tb, tc, tr, tma_store, t.cluster, args, epilogue, stream);
 }
 
 int gemm_bf16_fused(const bf16* A, int lda, const bf16* W, int ldw, void* out, int ldc, const float* bias,

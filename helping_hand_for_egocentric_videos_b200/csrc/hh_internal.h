@@ -120,9 +120,10 @@ int assemble_tokens_ln(const float* tok, const float* cls, const float* pos, con
 size_t attn_cls_workspace_bytes(int B, int T, int n, int H);
 int attn_space(const bf16* qkv, bf16* out, int B, int T, int n, int H, float* cls_ws, cudaStream_t stream);
 int attn_time(const bf16* qkv, bf16* out, int B, int T, int n, int H, float* cls_ws, cudaStream_t stream);
-// tcgen05/TMEM implementation of attn_space for n <= 256 (attn_space dispatches to it; HH_ATTN_SPACE_MMA_SYNC=1 disables)
+// attn_time for T <= 16 (attn_time_v2.cu)
 int attn_time_v2(const bf16* qkv, bf16* out, int B, int T, int n, int H, float* cls_ws, int pchunk, int nchunks,
                  cudaStream_t stream);
+// tcgen05/TMEM implementation of attn_space for n <= 256 (attn_space dispatches to it)
 bool attn_space_tc_supported(int n);
 int attn_space_tc(const bf16* qkv, bf16* out, int B, int T, int n, int H, float* cls_ws, cudaStream_t stream);
 int attn_cls_merge(const bf16* qkv, const float* parts, bf16* out, int B, int N, int H, int nparts, cudaStream_t stream);
@@ -146,7 +147,7 @@ struct LinArgs {
   DropCfg drop; uint32_t drop_site;       // training: dropout on act(x W^T + b) before the residual add, idx = row*N + col
 };
 int linear_f32(const LinArgs& a, cudaStream_t stream);          // lin3.cu (pipelined); shapes it refuses go to:
-int linear_f32_legacy(const LinArgs& a, cudaStream_t stream);   // decoder.cu (also with HH_LIN_LEGACY=1)
+int linear_f32_legacy(const LinArgs& a, cudaStream_t stream);   // decoder.cu
 // Query self-attention: q,k,v fp32 [B*Q, C] (q pre-scaled), heads of 64 -> out fp32 [B*Q, C].
 // drop: dropout on the attention probabilities (training), idx = ((b*heads + h)*Q + i)*Q + j
 int self_attn_queries(const float* q, const float* k, const float* v, int ld, float* out, int B, int Q, int heads,
@@ -229,7 +230,7 @@ int cross_attn_bwd(const float* q, const bf16* K, const bf16* V, int ldkv, const
                    DropCfg drop = drop_off(), uint32_t drop_site = 0,
                    const float* lse_saved = nullptr);   // the forward's lse_out; recomputed from q, K when absent
 // cross_attn_bwd.cu runs the tensor-core kernel; the first-generation SIMT statement (decoder_bwd.cu) serves unaligned
-// operands and HH_CROSS_BWD_SIMT=1
+// q / dO / dK / dV and dropout with S % 8 != 0
 size_t cross_attn_bwd_simt_workspace_bytes(int B, int Q, int heads, int S);
 int cross_attn_bwd_simt(const float* q, const bf16* K, const bf16* V, int ldkv, const float* O, const float* dO, float* dq,
                         bf16* dK, bf16* dV, int lddkv, int B, int Q, int heads, int S, void* workspace, cudaStream_t s,

@@ -86,14 +86,6 @@ __device__ __forceinline__ void tma_load_2d(const CUtensorMap* m, uint64_t* bar,
       ::"r"(smem_u32(dst)), "l"(reinterpret_cast<uint64_t>(m)), "r"(smem_u32(bar)), "r"(crd0), "r"(crd1)
       : "memory");
 }
-__device__ __forceinline__ void tma_load_2d_hint(const CUtensorMap* m, uint64_t* bar, void* dst, int crd0, int crd1,
-                                                 uint64_t policy) {
-  asm volatile(
-      "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes.L2::cache_hint"
-      " [%0], [%1, {%3, %4}], [%2], %5;"
-      ::"r"(smem_u32(dst)), "l"(reinterpret_cast<uint64_t>(m)), "r"(smem_u32(bar)), "r"(crd0), "r"(crd1), "l"(policy)
-      : "memory");
-}
 // Same, delivered to the same shared-memory offset of every CTA in `cta_mask` of the cluster; each destination CTA's
 // mbarrier at the same offset receives the complete_tx for the bytes written into that CTA.
 __device__ __forceinline__ void tma_load_2d_mcast(const CUtensorMap* m, uint64_t* bar, void* dst, int crd0, int crd1,
@@ -109,18 +101,6 @@ __device__ __forceinline__ void tma_store_2d(const CUtensorMap* m, uint32_t src_
   asm volatile("cp.async.bulk.tensor.2d.global.shared::cta.bulk_group [%0, {%2, %3}], [%1];"
                ::"l"(reinterpret_cast<uint64_t>(m)), "r"(src_smem), "r"(crd0), "r"(crd1)
                : "memory");
-}
-// Same with an L2 cache-policy operand (createpolicy): streaming data that nothing re-reads soon should not push the
-// operand tiles of the running GEMM out of L2.
-__device__ __forceinline__ void tma_store_2d_hint(const CUtensorMap* m, uint32_t src_smem, int crd0, int crd1, uint64_t policy) {
-  asm volatile("cp.async.bulk.tensor.2d.global.shared::cta.bulk_group.L2::cache_hint [%0, {%2, %3}], [%1], %4;"
-               ::"l"(reinterpret_cast<uint64_t>(m)), "r"(src_smem), "r"(crd0), "r"(crd1), "l"(policy)
-               : "memory");
-}
-__device__ __forceinline__ uint64_t l2_policy_evict_first() {
-  uint64_t p;
-  asm volatile("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;" : "=l"(p));
-  return p;
 }
 __device__ __forceinline__ uint64_t l2_policy_evict_last() {
   uint64_t p;

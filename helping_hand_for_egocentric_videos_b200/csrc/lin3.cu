@@ -16,8 +16,6 @@
 // prologues (query_pos add, ReLU, dropout mask and activation derivative of the incoming gradient) run in shared memory
 // on the 16-byte pieces each thread copied itself -- once per element instead of once per consuming warp, with one
 // Philox block per four dropout decisions.
-#include <cstdlib>
-
 #include "hh_internal.h"
 #include "hh_ptx.cuh"
 
@@ -26,10 +24,6 @@ namespace hh {
 namespace {
 
 constexpr int BM = 32, BN = 64, BK = 32, NST = 4;
-#ifndef HH_LIN3_CHAINS
-#define HH_LIN3_CHAINS 1   // accumulator sets the k-steps of a chunk alternate between; measured 1 > 2 > 4: registers (occupancy) matter more than MMA chain length
-#endif
-constexpr int NACC = HH_LIN3_CHAINS;
 constexpr int LDK = BK + 4;     // reduction-contiguous tiles [rows][36]: fragment loads (row g, column t) hit 32 banks
 constexpr int LDA_R = BM + 8;   // reduction-major A tile [32][40]: (row t, column g) -> bank 8 t + g
 constexpr int LDB_R = BN + 8;   // reduction-major B tile [32][72]
@@ -225,10 +219,11 @@ __global__ void __launch_bounds__(256) lin3_kernel(const Lin3Args a) {
     const float* Bs = As + off_b;
     // The tensor core truncates when it accumulates: chain only this chunk's 4 k-steps there (the two small correction
     // products in their own accumulator) and add the chunk's partial to the running sum with a rounded fp32 add.
-    // (even and odd k-steps in separate accumulators: dependent chains of 2 / 4 MMAs instead of 4 / 8)
-    float ph[NACC][2][4], pc[NACC][2][4];
+    // (One accumulator set: splitting the k-steps over 2 or 4 sets measured slower -- registers (occupancy) matter more
+    // than MMA chain length.)
+    float ph[2][4], pc[2][4];
 #pragma unroll
-    for (int i = 0; i < NACC * 8; ++i) (&ph[0][0][0])[i] = (&pc[0][0][0])[i] = 0.f;
+    for (int i = 0; i < 8; ++i) (&ph[0][0])[i] = (&pc[0][0])[i] = 0.f;
     // Forward (both tiles reduction-contiguous): the MMA's reduction index is a free permutation as long as A and B use
     // the same one -- thread t takes the chunk's elements 8t .. 8t+7 (k-step ks: 8t + 2ks as k = t, 8t + 2ks + 1 as
     // k = t + 4), so a fragment row is two 16-byte loads per chunk instead of eight 4-byte ones (rows of 36 floats:
@@ -269,20 +264,15 @@ __global__ void __launch_bounds__(256) lin3_kernel(const Lin3Args a) {
         uint32_t bh0, bl0, bh1, bl1;
         split_fast(b0, bh0, bl0);
         split_fast(b1, bh1, bl1);
-        mma_tf32_1688(pc[ks % NACC][j], al, bh0, bh1);
-        mma_tf32_1688(ph[ks % NACC][j], ah, bh0, bh1);
-        mma_tf32_1688(pc[ks % NACC][j], ah, bl0, bl1);
+        mma_tf32_1688(pc[j], al, bh0, bh1);
+        mma_tf32_1688(ph[j], ah, bh0, bh1);
+        mma_tf32_1688(pc[j], ah, bl0, bl1);
       }
     }
 #pragma unroll
     for (int j = 0; j < 2; ++j)
 #pragma unroll
-      for (int e = 0; e < 4; ++e) {
-        float hsum = ph[0][j][e], csum = pc[0][j][e];
-#pragma unroll
-        for (int i = 1; i < NACC; ++i) { hsum += ph[i][j][e]; csum += pc[i][j][e]; }
-        acc[j][e] += hsum + csum;
-      }
+      for (int e = 0; e < 4; ++e) acc[j][e] += ph[j][e] + pc[j][e];
     if (MODE == MODE_WGRAD && a.db && blockIdx.x == 0 && tid < BM) {
 #pragma unroll 8
       for (int r = 0; r < BK; ++r) bsum += As[r * LDA_R + tid];
@@ -334,14 +324,6 @@ __global__ void __launch_bounds__(256) lin3_kernel(const Lin3Args a) {
 
 inline bool al16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; }
 
-bool lin3_disabled() {
-  static const bool off = [] {
-    const char* e = std::getenv("HH_LIN_LEGACY");
-    return e && e[0] == '1';
-  }();
-  return off;
-}
-
 template <int MODE>
 int launch_lin3(const Lin3Args& a, int split, cudaStream_t s) {
   const size_t stage = A_FLOATS + B_FLOATS + (a.Ax ? A_FLOATS : 0) + (a.Bx ? B_FLOATS : 0);
@@ -366,8 +348,7 @@ int linear_f32(const LinArgs& a, cudaStream_t stream) {
   HH_REQUIRE(a.K % 4 == 0 && a.ldi % 4 == 0 && al16(a.in) && al16(a.W) && (a.in_add == nullptr || al16(a.in_add)),
              "linear_f32: input, weight and addend rows must be 16-byte aligned (K and ldi multiples of 4)");
   HH_REQUIRE(a.in_add == nullptr || a.add_mod > 0, "linear_f32: add_mod");
-  const bool ok = !lin3_disabled() && a.N % 2 == 0;
-  if (!ok) return linear_f32_legacy(a, stream);
+  if (a.N % 2 != 0) return linear_f32_legacy(a, stream);
   Lin3Args l{};
   l.A = a.in; l.lda = a.ldi; l.Ax = a.in_add; l.ldax = a.K; l.ax_mod = a.in_add ? a.add_mod : 1;
   l.B = a.W; l.ldb = a.K;
@@ -398,7 +379,7 @@ bool grad_operand_ok(const LinBwdArgs& a) {
 int linear_dgrad_f32(const LinBwdArgs& a, cudaStream_t s) {
   HH_REQUIRE(a.R > 0 && a.N > 0 && a.K > 0 && a.dY && a.W && a.dX, "linear_dgrad: bad argument");
   HH_REQUIRE(a.act == 0 || a.Y != nullptr, "linear_dgrad: activation derivative needs the saved output");
-  const bool ok = !lin3_disabled() && grad_operand_ok(a) && a.K % 4 == 0 && al16(a.W);
+  const bool ok = grad_operand_ok(a) && a.K % 4 == 0 && al16(a.W);
   if (!ok) return linear_dgrad_f32_legacy(a, s);
   Lin3Args l{};
   grad_operand(a, l);
@@ -411,7 +392,7 @@ int linear_dgrad_f32(const LinBwdArgs& a, cudaStream_t s) {
 int linear_wgrad_f32(const LinBwdArgs& a, cudaStream_t s) {
   HH_REQUIRE(a.R > 0 && a.N > 0 && a.K > 0 && a.dY && a.X && a.dW, "linear_wgrad: bad argument");
   HH_REQUIRE(a.act == 0 || a.Y != nullptr, "linear_wgrad: activation derivative needs the saved output");
-  const bool ok = !lin3_disabled() && grad_operand_ok(a) && a.K % 4 == 0 && a.ldx % 4 == 0 && al16(a.X) &&
+  const bool ok = grad_operand_ok(a) && a.K % 4 == 0 && a.ldx % 4 == 0 && al16(a.X) &&
                   (a.x_add == nullptr || (al16(a.x_add) && a.add_mod > 0));
   if (!ok) return linear_wgrad_f32_legacy(a, s);
   Lin3Args l{};
@@ -423,12 +404,8 @@ int linear_wgrad_f32(const LinBwdArgs& a, cudaStream_t s) {
   // partial tiles are combined with fp32 atomics (summation order, hence the last bits, vary from run to run).
   const int tiles = ((a.K + BN - 1) / BN) * ((a.N + BM - 1) / BM);
   int split = (4 * num_sms() + tiles - 1) / tiles;
-  static const int min_rows = [] {   // rows per CTA of the split (HH_LIN3_WGRAD_ROWS: A/B knob)
-    const char* e = std::getenv("HH_LIN3_WGRAD_ROWS");
-    const int v = e ? std::atoi(e) : 0;
-    return v >= 32 ? v : 128;
-  }();
-  const int max_split = (a.R + min_rows - 1) / min_rows;   // default: at least 128 rows (4 chunks: one full ring) per CTA
+  // at least 128 rows (4 chunks: one full ring) per CTA; 64 and 256 measured within noise of it
+  const int max_split = (a.R + 127) / 128;
   if (split > max_split) split = max_split;
   if (split > 64) split = 64;
   if (split < 1 || (a.beta != 0.f && a.beta != 1.f)) split = 1;

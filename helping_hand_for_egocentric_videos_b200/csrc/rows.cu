@@ -16,12 +16,8 @@ __global__ void __launch_bounds__(256) ln_rows_kernel(const LnArgs a) {
   if (warp_lin >= a.M) return;
   // Rows are walked from the END of the matrix: the GEMM that produced `delta` wrote its last row tiles last, so they
   // are still in the 126 MB L2, and the GEMM that follows reads the rows written last here (the first ones) first.
-  // Measured +0.5 ... 0.7 % clips/s with the same walk in the attention kernels (A/B on one box, HH_FORWARD_WALK build).
-#ifdef HH_FORWARD_WALK
-  const int warp = warp_lin;
-#else
+  // Measured +0.5 ... 0.7 % clips/s with the same walk in the attention kernels (A/B on one box against a forward walk).
   const int warp = a.M - 1 - warp_lin;
-#endif
   const int nv = a.D >> 7;  // float4 per lane
   const float* xr = a.x + static_cast<size_t>(warp) * a.ldx;
   float4 v[LN_MAX_VEC];

@@ -13,8 +13,6 @@
 #include "hh_ptx.cuh"
 #include "engine.h"
 
-#include <cstdlib>
-
 namespace hh {
 
 namespace {
@@ -145,8 +143,7 @@ static DevBuf g_sim_ws;
 
 int sim_matrix(const float* a, const float* b, float* out, int Na, int Nb, int d, float eps, cudaStream_t stream) {
   HH_REQUIRE(Na > 0 && Nb > 0 && d > 0, "sim_matrix: empty problem");
-  static const bool tc_ok = std::getenv("HH_SIM_SIMT") == nullptr;
-  if (tc_ok && Na >= 128 && Nb >= 128 && d % 8 == 0 && (reinterpret_cast<uintptr_t>(out) & 3) == 0) {
+  if (Na >= 128 && Nb >= 128 && d % 8 == 0 && (reinterpret_cast<uintptr_t>(out) & 3) == 0) {
     const size_t abytes = (static_cast<size_t>(Na) * 4 * d * 2 + 255) & ~size_t(255);
     const size_t bbytes = static_cast<size_t>(Nb) * 4 * d * 2;
     int rc = g_sim_ws.reserve(abytes + bbytes);

@@ -23,8 +23,9 @@ def _close(got, want, name, rtol=2e-5, atol=None):
 
 @pytest.mark.parametrize("R,N,K,act,add,in_relu", [(65, 512, 512, 0, True, False), (832, 2048, 512, 1, False, False),
                                                    (100, 4, 512, 2, False, False), (37, 256, 768, 0, False, True),
-                                                   (5, 40, 24, 1, True, False)])
+                                                   (5, 40, 24, 1, True, False), (70, 30, 64, 1, True, False)])
 def test_linear_backward(R, N, K, act, add, in_relu):
+    """N = 30 (not a multiple of 4) runs both gradients on the first-generation kernels instead of lin3_kernel."""
     g = torch.Generator().manual_seed(R + N)
     x = torch.randn(R, K, generator=g)
     w = torch.randn(N, K, generator=g) / K ** 0.5
@@ -92,6 +93,17 @@ def test_cross_attention_backward(B, Q, heads, S):
     _close(dq, q0.grad, "dq", 1e-4)
     _close(dK, K0.grad, "dK", 2 ** -7, atol=1e-4)
     _close(dV, V0.grad, "dV", 2 ** -7, atol=1e-4)
+    # q and dO 4 bytes off an 8-byte boundary: the tensor-core kernel does not take them, the SIMT kernels do
+    def off8(t):
+        flat = torch.empty(t.numel() + 1, device="cuda")
+        flat[1:] = t.flatten().cuda()
+        return flat[1:].view(t.shape)
+    qu, dOu = off8(q), off8(dO)
+    assert qu.data_ptr() % 8 != 0 and dOu.data_ptr() % 8 != 0
+    dq, dK, dV = _ops().cross_attention_backward(qu, K.cuda(), V.cuda(), O.detach().cuda(), dOu, B, Q, heads, S)
+    _close(dq, q0.grad, "dq (SIMT)", 1e-4)
+    _close(dK, K0.grad, "dK (SIMT)", 2 ** -7, atol=1e-4)
+    _close(dV, V0.grad, "dV (SIMT)", 2 ** -7, atol=1e-4)
 
 
 # ------------------------------------------------------------------------------------------ whole-decoder backward

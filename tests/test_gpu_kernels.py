@@ -117,8 +117,10 @@ def _ref_attention(qkv, B, T, n, H, mode):
 
 
 @pytest.mark.parametrize("B,T,n,H", [(2, 3, 16, 2), (1, 4, 196, 12), (2, 16, 256, 2), (1, 4, 256, 16), (3, 1, 4, 1),
-                                     (1, 2, 50, 3), (1, 32, 16, 4), (1, 8, 64, 5)])
+                                     (1, 2, 50, 3), (1, 32, 16, 4), (1, 8, 64, 5), (1, 2, 300, 2)])
 def test_divided_attention(B, T, n, H):
+    """n > 256 runs the spatial mma.sync kernel instead of the tcgen05 one; T other than 4 / 8 / 16 runs the runtime-T
+    temporal kernel, T > 16 the SIMT one."""
     ops = _ops()
     N = 1 + T * n
     qkv = _rand(B * N, 3 * H * 64, seed=20, scale=1.0)

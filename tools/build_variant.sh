@@ -1,6 +1,6 @@
 #!/bin/bash
 # A/B helper: build a variant of libhh_b200.so with extra -D flags on selected sources.
-#   tools/build_variant.sh NAME "-DHH_SCALAR_EPI" gemm_tcgen05.cu [more.cu ...]
+#   tools/build_variant.sh NAME "-DHH_GEMM_TRACE" gemm_tcgen05.cu [more.cu ...]
 # -> tools/ab/libhh_b200_NAME.so (git-ignored, travels with gpurun); run with HH_B200_LIB=tools/ab/libhh_b200_NAME.so
 set -e
 ROOT=$(cd "$(dirname "$0")/.." && pwd)

@@ -1,6 +1,5 @@
 """Times the small fp32 linear family (forward, data gradient, weight gradient) at the decoder's shapes.
-  python tools/time_lin3.py            (HH_LIN_LEGACY=1 python tools/time_lin3.py for the first-generation kernels)"""
-import os
+  python tools/time_lin3.py"""
 import sys
 
 import torch
@@ -23,7 +22,6 @@ def gpu_us(fn, iters=30, warm=5):
 
 
 def main():
-    print("HH_LIN_LEGACY =", os.environ.get("HH_LIN_LEGACY", "0"))
     for R, N, K in [(832, 256, 256), (832, 512, 256), (832, 2048, 256), (832, 256, 2048), (19968, 256, 256), (4992, 256, 256),
                     (65, 256, 256), (19968, 4, 256)]:
         x = torch.randn(R, K, device="cuda")

@@ -1,5 +1,5 @@
-"""GEMM timing at the EgoMCQ question shape (5 clips x 4 frames: M = 5125 rows) for the tile-width rule A/B.
-  python tools/time_small_m.py ; HH_GEMM_NO_WAVE_RULE=1 python tools/time_small_m.py"""
+"""GEMM timing at the EgoMCQ question shape (5 clips x 4 frames: M = 5125 rows; another M as the first argument).
+  python tools/time_small_m.py [M]"""
 import os
 import sys
 
@@ -26,4 +26,4 @@ for name, N, K, epi in (("qkv", 3072, 1024, 0), ("proj", 1024, 1024, 0), ("fc1",
     torch.cuda.synchronize()
     us = e0.elapsed_time(e1) * 1e3 / 50
     res[name] = (round(us, 1), round(2.0 * M * N * K / us / 1e6))
-print("wave rule", "off" if os.environ.get("HH_GEMM_NO_WAVE_RULE") else "on", res, "(us, TFLOP/s)")
+print("M", M, res, "(us, TFLOP/s)")
