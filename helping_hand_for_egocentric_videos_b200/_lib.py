@@ -58,6 +58,7 @@ SIGNATURES = {
     "hh_decoder_backward_checked": (_i, [_p, C.c_uint64, _p, _p, _p, _p, _p]),
     "hh_decoder_get_grad": (_i, [_p, C.c_char_p, _p, _i64, _p]),
     "hh_decoder_get_grads": (_i, [_p, _p, _p, _i, _p, _i64, _p]),
+    "hh_decoder_get_saved": (_i, [_p, C.c_char_p, _i, _p, _i64, _p]),
     "hh_decoder_set_weights": (_i, [_p, _p, _p, _p, _i, _p]),
     "hh_decoder_flops_per_clip": (C.c_double, [_p, _i]),
     "hh_decoder_last_launches": (_i, [_p]),

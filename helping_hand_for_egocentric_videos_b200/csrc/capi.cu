@@ -191,6 +191,51 @@ int hh_decoder_get_grad(hh_decoder* dec, const char* key, float* out, int64_t nu
   return 0;
   HH_GUARD_END
 }
+int hh_decoder_get_saved(hh_decoder* dec, const char* name, int layer, void* out, int64_t bytes, void* stream) {
+  HH_GUARD_BEGIN
+  if (!dec || !name || !out) return fail(-2, "hh_decoder_get_saved: null argument");
+  const Decoder& d = dec->impl;
+  if (d.saved_B <= 0 || d.saved.empty())
+    return fail(-2, "hh_decoder_get_saved: no training forward since the last forward");
+  const int C = d.cfg.d_model, Lr = d.cfg.num_layers, Q = d.cfg.num_queries, T = d.saved_T;
+  const int64_t B = d.saved_B, R = B * Q, BS = B * T * d.cfg.patches_per_frame;
+  const bool traj = d.cfg.pred_traj && T == d.cfg.num_frames;
+  const int64_t rows_box = static_cast<int64_t>(Lr) * R * (traj ? T : 1);
+  const std::string nm(name);
+  const void* src = nullptr;
+  int64_t want = 0;
+  if (layer == -1) {
+    const void* const bufs[] = {d.ws_memf.ptr, d.ws_mem.ptr, d.ws_mempos.ptr, d.ws_k.ptr, d.ws_v.ptr, d.sv_x1, d.sv_x2,
+                                traj ? d.sv_cond : nullptr};
+    const char* const names[] = {"memf", "mem", "mempos", "k", "v", "box_x1", "box_x2", "cond"};
+    const int64_t sizes[] = {BS * C * 4, BS * C * 2, BS * C * 2, BS * Lr * C * 2, BS * Lr * C * 2, rows_box * C * 4,
+                             rows_box * C * 4, rows_box * C * 4};
+    for (int j = 0; j < 8; ++j)
+      if (nm == names[j]) {
+        src = bufs[j];
+        want = sizes[j];
+      }
+    if (!src) return fail(-2, "hh_decoder_get_saved: unknown memory-side / head buffer '" + nm + "'");
+  } else {
+    if (layer < 0 || layer >= Lr)
+      return fail(-2, "hh_decoder_get_saved: layer " + std::to_string(layer) + " out of range [0, " + std::to_string(Lr) + ")");
+    const Decoder::LayerBufs& A = d.saved[layer];
+    const float* const bufs[] = {A.x0, A.x1, A.x2, A.x3, A.n1, A.n2, A.n3, A.qkv, A.o1, A.qc, A.o2, A.f, A.lse};
+    const char* const names[] = {"x0", "x1", "x2", "x3", "n1", "n2", "n3", "qkv", "o1", "qc", "o2", "f", "lse"};
+    const int64_t widths[] = {C, C, C, C, C, C, C, 3 * C, C, C, C, d.cfg.dim_feedforward, 0};
+    for (int j = 0; j < 13; ++j)
+      if (nm == names[j]) {
+        src = bufs[j];
+        want = (j == 12 ? B * d.cfg.nhead * Q : R * widths[j]) * 4;
+      }
+    if (!src) return fail(-2, "hh_decoder_get_saved: unknown per-layer buffer '" + nm + "'");
+  }
+  if (bytes != want)
+    return fail(-2, "hh_decoder_get_saved: '" + nm + "' is " + std::to_string(want) + " bytes, got " + std::to_string(bytes));
+  HH_CHECK_CUDA(cudaMemcpyAsync(out, src, static_cast<size_t>(want), cudaMemcpyDeviceToDevice, S(stream)));
+  return 0;
+  HH_GUARD_END
+}
 int hh_decoder_get_grads(hh_decoder* dec, const char* const* keys, const int64_t* numels, int n, float* out, int64_t total,
                          void* stream) {
   HH_GUARD_BEGIN

@@ -136,6 +136,13 @@ uint64_t hh_decoder_generation(const hh_decoder* dec);
 int hh_decoder_backward_checked(hh_decoder* dec, uint64_t generation, const float* hs, const float* boxes,
                                 const float* d_hs, const float* d_boxes, void* stream);
 int hh_decoder_get_grad(hh_decoder* dec, const char* key, float* out, int64_t numel, void* stream);
+/* Copy a buffer the last training forward saved into `out` (device memory, `bytes` long).  Per layer (0 <= layer < L):
+ * "x0".."x3", "n1".."n3", "qkv", "o1", "qc", "o2", "f" (fp32 [B*Q, .]), "lse" (fp32 [B*heads, Q]).  layer = -1:
+ * "memf" (fp32 [B*S, C]), "mem", "mempos" (bf16 [B*S, C]), "k", "v" (bf16 [B*S, L*C]), "box_x1", "box_x2", "cond"
+ * (fp32 [rows_box, C]; "cond" only with the trajectory head).  Refuses (-2) an unknown name, a layer out of range, a
+ * byte count that does not match, and any call after an inference forward (it shares one buffer set between layers).
+ * For tests and diagnostics. */
+int hh_decoder_get_saved(hh_decoder* dec, const char* name, int layer, void* out, int64_t bytes, void* stream);
 /* Batched forms (one call per training step instead of one per parameter: the step's 135 keys made the Python side of
  * the backward host-bound).  get_grads packs the gradients of keys[0..n) back to back into `out` (`total` = sum of
  * numels); set_weights is hh_decoder_set_weight over n (key, data, numel) triples. */
