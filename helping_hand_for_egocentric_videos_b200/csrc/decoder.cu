@@ -1,6 +1,6 @@
 // Query-side kernels of the object-aware decoder (model/tfm_decoder.py).  The decoder's heavy contractions (memory
 // projection, the 6 layers' K/V projections, the class head) run on the tcgen05 GEMM; what is left operates on the
-// Q <= 16 learned queries per clip and is latency-, not FLOP-bound.  Everything here is fp32.
+// Q <= kMaxQueries (32) learned queries per clip and is latency-, not FLOP-bound.  Everything here is fp32.
 //
 //   linear_f32          small-M nn.Linear (+ query_pos add on the input, bias, ReLU/sigmoid, residual); fp32 operands on
 //                       the tensor cores as error-compensated TF32 (3 MMAs per product, fp32-level accuracy)
@@ -112,11 +112,13 @@ __global__ void __launch_bounds__(256) linear_f32_kernel(const LinArgs a) {
 }
 
 // ------------------------------------------------------------------------------------------ self attention
+// one warp per (clip, head), lane = query: a warp holds every query the decoder takes; terms for j >= Q are exact zeros
+static_assert(kMaxQueries <= 32, "self_attn_kernel: one lane per query");
 __global__ void __launch_bounds__(32)
 self_attn_kernel(const float* __restrict__ q, const float* __restrict__ k, const float* __restrict__ v, int ld,
                  float* __restrict__ out, int Q, int heads, DropCfg drop, uint32_t drop_site) {
-  __shared__ float Ks[16][HD + 1];
-  __shared__ float Vs[16][HD + 1];
+  __shared__ float Ks[kMaxQueries][HD + 1];
+  __shared__ float Vs[kMaxQueries][HD + 1];
   const int h = blockIdx.x % heads, b = blockIdx.x / heads;
   const int lane = threadIdx.x;
   const int C = heads * HD;
@@ -128,10 +130,10 @@ self_attn_kernel(const float* __restrict__ q, const float* __restrict__ k, const
   __syncwarp();
   if (lane >= Q) return;
   const float* qr = q + static_cast<size_t>(b * Q + lane) * ld + h * HD;
-  float s[16];
+  float s[kMaxQueries];
   float mx = -INFINITY;
 #pragma unroll
-  for (int j = 0; j < 16; ++j) {
+  for (int j = 0; j < kMaxQueries; ++j) {
     if (j < Q) {
       float acc = 0.f;
       for (int d = 0; d < HD; ++d) acc += qr[d] * Ks[j][d];
@@ -143,7 +145,7 @@ self_attn_kernel(const float* __restrict__ q, const float* __restrict__ k, const
   }
   float l = 0.f;
 #pragma unroll
-  for (int j = 0; j < 16; ++j) {
+  for (int j = 0; j < kMaxQueries; ++j) {
     s[j] = exp2f((s[j] - mx) * LOG2E);
     l += s[j];
   }
@@ -151,21 +153,21 @@ self_attn_kernel(const float* __restrict__ q, const float* __restrict__ k, const
   if (drop.thr) {  // dropout on the normalised probabilities (nn.MultiheadAttention, training mode)
     const uint64_t base = (static_cast<uint64_t>(blockIdx.x) * Q + lane) * Q;
 #pragma unroll
-    for (int j = 0; j < 16; ++j)
+    for (int j = 0; j < kMaxQueries; ++j)
       if (j < Q) s[j] *= drop_mult(drop, drop_site, base + j);
   }
   float* o = out + static_cast<size_t>(b * Q + lane) * C + h * HD;
   for (int d = 0; d < HD; ++d) {
     float acc = 0.f;
 #pragma unroll
-    for (int j = 0; j < 16; ++j)
+    for (int j = 0; j < kMaxQueries; ++j)
       if (j < Q) acc += s[j] * Vs[j][d];
     o[d] = acc * inv;
   }
 }
 
 // ------------------------------------------------------------------------------------------ cross attention
-constexpr int XQ = 16;       // max queries
+constexpr int XQ = 16;       // max queries of this differential-test statement (static smem: 48 KB at 16)
 constexpr int XWARPS = 4;
 constexpr int XPART = HD + 2;  // per (query): m, l, o[64]
 
@@ -378,7 +380,7 @@ int linear_f32_legacy(const LinArgs& a, cudaStream_t stream) {
 
 int self_attn_queries(const float* q, const float* k, const float* v, int ld, float* out, int B, int Q, int heads,
                       cudaStream_t stream, DropCfg drop, uint32_t drop_site) {
-  HH_REQUIRE(Q >= 1 && Q <= 16, "self_attn_queries: 1..16 queries supported");
+  HH_REQUIRE(Q >= 1 && Q <= kMaxQueries, "self_attn_queries: 1..32 queries supported");
   self_attn_kernel<<<B * heads, 32, 0, stream>>>(q, k, v, ld, out, Q, heads, drop, drop_site);
   HH_CHECK_LAUNCH("self_attn_kernel");
   return 0;
@@ -389,7 +391,8 @@ size_t cross_attn_simt_workspace_bytes(int B, int Q, int heads, int S) {
   return static_cast<size_t>(B) * heads * cross_splits(B, heads, S) * XQ * XPART * sizeof(float);
 }
 
-// fp32 SIMT statement of the cross attention (kept as a second implementation for differential tests)
+// fp32 SIMT statement of the cross attention (kept as a second implementation for differential tests; Q <= 16 only,
+// tests compare larger Q with float64 torch)
 int cross_attn_simt(const float* q, const bf16* K, const bf16* V, int ldkv, float* out, int B, int Q, int heads, int S,
                     void* workspace, cudaStream_t stream) {
   HH_REQUIRE(Q >= 1 && Q <= XQ, "cross_attn: 1..16 queries supported");

@@ -1,6 +1,6 @@
 // Backward primitives of the object-aware decoder (SURVEY.md section 8f row 2: "decoder / heads backward").
-// The query side (Q <= 16 rows per clip) keeps fp32 operands like its forward (linears as error-compensated TF32 on the
-// tensor cores, the rest SIMT); the memory side (B*S patch tokens) reuses
+// The query side (Q <= kMaxQueries = 32 rows per clip) keeps fp32 operands like its forward (linears as
+// error-compensated TF32 on the tensor cores, the rest SIMT); the memory side (B*S patch tokens) reuses
 // the tcgen05 GEMM for its data- and weight-gradient contractions (engine_bwd.cu) and needs from here only the
 // cross-attention backward, LayerNorm backward, column sums and transposes.
 //
@@ -293,12 +293,13 @@ __global__ void reduce_parts_kernel(const float* __restrict__ part, int P, int n
 
 // ------------------------------------------------------------------------------------------ self-attention backward
 // one warp per (clip, head); lane i = query row i
+static_assert(kMaxQueries <= 32, "self_attn_bwd_kernel: one lane per query");
 __global__ void __launch_bounds__(32)
 self_attn_bwd_kernel(const float* __restrict__ q, const float* __restrict__ k, const float* __restrict__ v, int ld,
                      const float* __restrict__ dO, float* __restrict__ dq, float* __restrict__ dk, float* __restrict__ dv,
                      int ldg, int Q, int heads, DropCfg drop, uint32_t drop_site) {
-  __shared__ float Qs[16][HD + 1], Ks[16][HD + 1], Vs[16][HD + 1], Gs[16][HD + 1];
-  __shared__ float Ps[16][17], Ss[16][17];
+  __shared__ float Qs[kMaxQueries][HD + 1], Ks[kMaxQueries][HD + 1], Vs[kMaxQueries][HD + 1], Gs[kMaxQueries][HD + 1];
+  __shared__ float Ps[kMaxQueries][kMaxQueries + 1], Ss[kMaxQueries][kMaxQueries + 1];
   const int h = blockIdx.x % heads, b = blockIdx.x / heads;
   const int lane = threadIdx.x;
   for (int i = lane; i < Q * HD; i += 32) {
@@ -311,7 +312,7 @@ self_attn_bwd_kernel(const float* __restrict__ q, const float* __restrict__ k, c
   }
   __syncwarp();
   if (lane < Q) {
-    float s[16], mx = -INFINITY;
+    float s[kMaxQueries], mx = -INFINITY;
     for (int j = 0; j < Q; ++j) {
       float acc = 0.f;
       for (int d = 0; d < HD; ++d) acc += Qs[lane][d] * Ks[j][d];
@@ -325,7 +326,7 @@ self_attn_bwd_kernel(const float* __restrict__ q, const float* __restrict__ k, c
     }
     const float inv = 1.f / l;
     // with dropout (training): O = sum_j (m_j p_j) v_j, m_j in {0, 1/(1-p)}: dP_j = m_j (dO . v_j), dV_j gets m_j p_j dO
-    float dp[16], mult[16], Dsum = 0.f;
+    float dp[kMaxQueries], mult[kMaxQueries], Dsum = 0.f;
     for (int j = 0; j < Q; ++j) {
       s[j] *= inv;
       mult[j] = drop.thr ? drop_mult(drop, drop_site, (static_cast<uint64_t>(blockIdx.x) * Q + lane) * Q + j) : 1.f;
@@ -362,39 +363,42 @@ self_attn_bwd_kernel(const float* __restrict__ q, const float* __restrict__ k, c
 }
 
 // ------------------------------------------------------------------------------------------ cross-attention backward
-// (i) per (clip, head): lse_i over the S keys -- only when the forward did not keep it (cross_attn's lse_out).  Warp i owns
-// query row i; lanes stride over keys.
-__global__ void __launch_bounds__(512)
+// (i) per (clip, head): lse_i over the S keys -- only when the forward did not keep it (cross_attn's lse_out).  Up to 16
+// warps; warp w owns query rows w, w + warps, ...; lanes stride over keys.
+constexpr int kStatsWarps = 16;
+__global__ void __launch_bounds__(kStatsWarps * 32)
 cross_stats_kernel(const float* __restrict__ q, const bf16* __restrict__ K, int ldkv, float* __restrict__ lse, int Q,
                    int heads, int S) {
-  __shared__ float qs[16][HD];
+  __shared__ float qs[kMaxQueries][HD];
   const int h = blockIdx.x % heads, b = blockIdx.x / heads;
   const int C = heads * HD;
-  const int tid = threadIdx.x, i = tid >> 5, lane = tid & 31;
+  const int tid = threadIdx.x, lane = tid & 31;
   for (int e = tid; e < Q * HD; e += blockDim.x) qs[e / HD][e % HD] = q[static_cast<size_t>(b * Q + e / HD) * C + h * HD + e % HD];
   __syncthreads();
-  float m = -INFINITY, sacc = 0.f;
-  for (int j = lane; j < S; j += 32) {
-    const uint4* kr = reinterpret_cast<const uint4*>(K + (static_cast<size_t>(b) * S + j) * ldkv + h * HD);
-    float sc = 0.f;
+  for (int i = tid >> 5; i < Q; i += blockDim.x >> 5) {
+    float m = -INFINITY, sacc = 0.f;
+    for (int j = lane; j < S; j += 32) {
+      const uint4* kr = reinterpret_cast<const uint4*>(K + (static_cast<size_t>(b) * S + j) * ldkv + h * HD);
+      float sc = 0.f;
 #pragma unroll
-    for (int c = 0; c < 8; ++c) {
-      const uint4 u = kr[c];
-      const float2 a0 = unpack_bf16x2(u.x), a1 = unpack_bf16x2(u.y), a2 = unpack_bf16x2(u.z), a3 = unpack_bf16x2(u.w);
-      const float* qq = &qs[i][c * 8];
-      sc += qq[0] * a0.x + qq[1] * a0.y + qq[2] * a1.x + qq[3] * a1.y + qq[4] * a2.x + qq[5] * a2.y + qq[6] * a3.x + qq[7] * a3.y;
+      for (int c = 0; c < 8; ++c) {
+        const uint4 u = kr[c];
+        const float2 a0 = unpack_bf16x2(u.x), a1 = unpack_bf16x2(u.y), a2 = unpack_bf16x2(u.z), a3 = unpack_bf16x2(u.w);
+        const float* qq = &qs[i][c * 8];
+        sc += qq[0] * a0.x + qq[1] * a0.y + qq[2] * a1.x + qq[3] * a1.y + qq[4] * a2.x + qq[5] * a2.y + qq[6] * a3.x + qq[7] * a3.y;
+      }
+      const float nm = fmaxf(m, sc);
+      sacc = sacc * __expf(m - nm) + __expf(sc - nm);
+      m = nm;
     }
-    const float nm = fmaxf(m, sc);
-    sacc = sacc * __expf(m - nm) + __expf(sc - nm);
-    m = nm;
+    for (int o = 16; o; o >>= 1) {
+      const float om = __shfl_xor_sync(0xffffffffu, m, o), os = __shfl_xor_sync(0xffffffffu, sacc, o);
+      const float nm = fmaxf(m, om);
+      sacc = (m == -INFINITY ? 0.f : sacc * __expf(m - nm)) + (om == -INFINITY ? 0.f : os * __expf(om - nm));
+      m = nm;
+    }
+    if (lane == 0) lse[(static_cast<size_t>(b) * heads + h) * Q + i] = m + logf(sacc);
   }
-  for (int o = 16; o; o >>= 1) {
-    const float om = __shfl_xor_sync(0xffffffffu, m, o), os = __shfl_xor_sync(0xffffffffu, sacc, o);
-    const float nm = fmaxf(m, om);
-    sacc = (m == -INFINITY ? 0.f : sacc * __expf(m - nm)) + (om == -INFINITY ? 0.f : os * __expf(om - nm));
-    m = nm;
-  }
-  if (lane == 0) lse[(static_cast<size_t>(b) * heads + h) * Q + i] = m + logf(sacc);
 }
 
 // (ii) one thread per key: p_ij, dS_ij, dV_j = sum_i p_ij dO_i, dK_j = sum_i dS_ij q_i;  D_i = dO_i . O_i is recomputed by
@@ -404,8 +408,8 @@ cross_keys_kernel(const float* __restrict__ q, const bf16* __restrict__ K, const
                   const float* __restrict__ dO, const float* __restrict__ O, const float* __restrict__ lse,
                   bf16* __restrict__ dK, bf16* __restrict__ dV, int lddkv, float* __restrict__ dS, int Q, int heads, int S,
                   DropCfg drop, uint32_t drop_site) {
-  __shared__ float qs[16][HD], gs[16][HD];
-  __shared__ float ls[16], ds_[16];
+  __shared__ float qs[kMaxQueries][HD], gs[kMaxQueries][HD];
+  __shared__ float ls[kMaxQueries], ds_[kMaxQueries];
   const int h = blockIdx.y % heads, b = blockIdx.y / heads;
   const int C = heads * HD;
   for (int i = threadIdx.x; i < Q * HD; i += blockDim.x) {
@@ -424,7 +428,7 @@ cross_keys_kernel(const float* __restrict__ q, const bf16* __restrict__ K, const
   const int j = blockIdx.x * blockDim.x + threadIdx.x;
   if (j >= S) return;
   const size_t rowoff = (static_cast<size_t>(b) * S + j);
-  float p[16], dsv[16];
+  float p[kMaxQueries], dsv[kMaxQueries];
   {
     float kf[HD], vf[HD];
     const uint4* kr = reinterpret_cast<const uint4*>(K + rowoff * ldkv + h * HD);
@@ -441,7 +445,7 @@ cross_keys_kernel(const float* __restrict__ q, const bf16* __restrict__ K, const
       vf[c * 8 + 4] = a2.x; vf[c * 8 + 5] = a2.y; vf[c * 8 + 6] = a3.x; vf[c * 8 + 7] = a3.y;
     }
 #pragma unroll
-    for (int i = 0; i < 16; ++i) {
+    for (int i = 0; i < kMaxQueries; ++i) {
       p[i] = dsv[i] = 0.f;
       if (i < Q) {
         float s = 0.f, dp = 0.f;
@@ -465,7 +469,7 @@ cross_keys_kernel(const float* __restrict__ q, const bf16* __restrict__ K, const
   for (int d = 0; d < HD; d += 2) {
     float v0 = 0.f, v1 = 0.f, k0 = 0.f, k1 = 0.f;
 #pragma unroll
-    for (int i = 0; i < 16; ++i)
+    for (int i = 0; i < kMaxQueries; ++i)
       if (i < Q) {
         v0 += p[i] * gs[i][d];
         v1 += p[i] * gs[i][d + 1];
@@ -481,22 +485,22 @@ cross_keys_kernel(const float* __restrict__ q, const bf16* __restrict__ K, const
 __global__ void __launch_bounds__(256)
 cross_dq_kernel(const float* __restrict__ dS, const bf16* __restrict__ K, int ldkv, float* __restrict__ dq, int Q, int heads,
                 int S) {
-  __shared__ float part[4][16][HD];
+  __shared__ float part[4][kMaxQueries][HD];
   const int h = blockIdx.x % heads, b = blockIdx.x / heads;
   const int C = heads * HD;
   const int d = threadIdx.x & 63, grp = threadIdx.x >> 6;  // 4 key groups x 64 dims
-  float acc[16];
+  float acc[kMaxQueries];
 #pragma unroll
-  for (int i = 0; i < 16; ++i) acc[i] = 0.f;
+  for (int i = 0; i < kMaxQueries; ++i) acc[i] = 0.f;
   const float* ds = dS + (static_cast<size_t>(b) * heads + h) * Q * S;
   for (int j = grp; j < S; j += 4) {
     const float kv = __bfloat162float(K[(static_cast<size_t>(b) * S + j) * ldkv + h * HD + d]);
 #pragma unroll
-    for (int i = 0; i < 16; ++i)
+    for (int i = 0; i < kMaxQueries; ++i)
       if (i < Q) acc[i] += ds[static_cast<size_t>(i) * S + j] * kv;
   }
 #pragma unroll
-  for (int i = 0; i < 16; ++i) part[grp][i][d] = acc[i];
+  for (int i = 0; i < kMaxQueries; ++i) part[grp][i][d] = acc[i];
   __syncthreads();
   for (int idx = threadIdx.x; idx < Q * HD; idx += 256) {
     const int i = idx / HD, dd = idx - i * HD;
@@ -654,7 +658,7 @@ int ln_backward_rows(const LnBwdArgs& a, cudaStream_t s) {
 
 int self_attn_bwd(const float* q, const float* k, const float* v, int ld, const float* dO, float* dq, float* dk, float* dv,
                   int ldg, int B, int Q, int heads, cudaStream_t s, DropCfg drop, uint32_t drop_site) {
-  HH_REQUIRE(B > 0 && Q >= 1 && Q <= 16 && heads > 0, "self_attn_bwd: 1..16 queries");
+  HH_REQUIRE(B > 0 && Q >= 1 && Q <= kMaxQueries && heads > 0, "self_attn_bwd: 1..32 queries");
   self_attn_bwd_kernel<<<B * heads, 32, 0, s>>>(q, k, v, ld, dO, dq, dk, dv, ldg, Q, heads, drop, drop_site);
   HH_CHECK_LAUNCH("self_attn_bwd_kernel");
   return 0;
@@ -665,7 +669,8 @@ size_t cross_attn_bwd_simt_workspace_bytes(int B, int Q, int heads, int S) {
 }
 
 int cross_lse(const float* q, const bf16* K, int ldkv, float* lse, int B, int Q, int heads, int S, cudaStream_t s) {
-  cross_stats_kernel<<<B * heads, 32 * Q, 0, s>>>(q, K, ldkv, lse, Q, heads, S);
+  HH_REQUIRE(Q >= 1 && Q <= kMaxQueries, "cross_lse: 1..32 queries");
+  cross_stats_kernel<<<B * heads, 32 * (Q < kStatsWarps ? Q : kStatsWarps), 0, s>>>(q, K, ldkv, lse, Q, heads, S);
   HH_CHECK_LAUNCH("cross_stats_kernel");
   return 0;
 }
@@ -673,11 +678,12 @@ int cross_lse(const float* q, const bf16* K, int ldkv, float* lse, int B, int Q,
 int cross_attn_bwd_simt(const float* q, const bf16* K, const bf16* V, int ldkv, const float* O, const float* dO, float* dq,
                         bf16* dK, bf16* dV, int lddkv, int B, int Q, int heads, int S, void* workspace, cudaStream_t s,
                         DropCfg drop, uint32_t drop_site, const float* lse_saved) {
+  HH_REQUIRE(B > 0 && Q >= 1 && Q <= kMaxQueries && heads > 0 && S > 0, "cross_attn_bwd: 1..32 queries");
   float* lse_ws = static_cast<float*>(workspace);
   float* dS = lse_ws + static_cast<size_t>(B) * heads * Q;
   const float* lse = lse_saved;
   if (lse == nullptr) {
-    cross_stats_kernel<<<B * heads, 32 * Q, 0, s>>>(q, K, ldkv, lse_ws, Q, heads, S);
+    if (int rc = cross_lse(q, K, ldkv, lse_ws, B, Q, heads, S, s)) return rc;
     lse = lse_ws;
   }
   dim3 grid((S + 127) / 128, B * heads);

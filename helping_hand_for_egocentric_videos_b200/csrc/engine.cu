@@ -476,7 +476,8 @@ Decoder::Decoder(const hh_decoder_cfg& c) : cfg(c) {
 int Decoder::validate(const hh_decoder_cfg& c) {
   HH_REQUIRE(c.d_model % 128 == 0 && c.d_model <= 1024, "decoder: d_model must be a multiple of 128, <= 1024");
   HH_REQUIRE(c.nhead > 0 && c.d_model == c.nhead * 64, "decoder: head dim must be 64");
-  HH_REQUIRE(c.num_queries >= 1 && c.num_queries <= 16, "decoder: 1..16 queries (num_queries==1 n_decode path unsupported)");
+  HH_REQUIRE(c.num_queries >= 1 && c.num_queries <= kMaxQueries,
+             "decoder: 1..32 queries (num_queries==1 n_decode path unsupported)");
   HH_REQUIRE(c.num_layers >= 1 && c.dim_feedforward % 32 == 0, "decoder: layers / ffn");
   HH_REQUIRE(c.feature_dim % 8 == 0 && c.num_classes1 >= 1, "decoder: feature_dim must be a multiple of 8");
   HH_REQUIRE(c.num_frames >= 1 && c.patches_per_frame >= 1, "decoder: frames / patches");

@@ -134,6 +134,10 @@ int attn_cls(const bf16* qkv, bf16* out, int B, int N, int H, cudaStream_t strea
 int attn_causal(const bf16* qkv, bf16* out, int G, int L, int H, cudaStream_t stream);
 
 // ---------------------------------------------------------------- decoder satellites (decoder.cu)
+// Most learned queries per clip the decoder takes (ObjDecoder num_queries = nq + 1).  Every query-side array, tile and
+// workspace size is derived from it: one warp lane per query in the self attention, two 16-row query blocks in the
+// tensor-core cross-attention kernels.
+constexpr int kMaxQueries = 32;
 // Small-M fp32 linear: out[R,N] = act((in[R,K] (+ in_add[r % add_mod, K])) * W[N,K]^T + bias) (+ residual[R,N]).
 struct LinArgs {
   const float* in; int ldi;
@@ -159,6 +163,7 @@ size_t cross_attn_workspace_bytes(int B, int Q, int heads, int S);
 int cross_attn(const float* q, const bf16* K, const bf16* V, int ldkv, float* out, int B, int Q, int heads, int S,
                void* workspace, cudaStream_t stream, DropCfg drop = drop_off(), uint32_t drop_site = 0,
                float* lse_out = nullptr);   // lse_out: optional fp32 [B*heads, Q] row log-sum-exp for cross_attn_bwd
+// fp32 SIMT statement of cross_attn for differential tests: Q <= 16 only
 size_t cross_attn_simt_workspace_bytes(int B, int Q, int heads, int S);
 int cross_attn_simt(const float* q, const bf16* K, const bf16* V, int ldkv, float* out, int B, int Q, int heads, int S,
                     void* workspace, cudaStream_t stream);

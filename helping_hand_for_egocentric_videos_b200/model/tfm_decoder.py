@@ -202,7 +202,8 @@ class Cross_Attention(nn.Module):
 
 
 class ObjDecoder(_DirtyHooks, nn.Module):
-    """Reference :111-241."""
+    """Reference :111-241.  num_queries (the scripts pass `--num_queries` + 1) may be 2 .. 32, in inference and in
+    training; 1 (the reference's n_decode = 10 branch) raises NotImplementedError, above 32 hh_decoder_create refuses."""
 
     def __init__(self, transformer, num_classes, num_queries, feature_dim=768, aux_loss=False, pred_traj=True,
                  num_frames=4, patches_per_frame=256, backbone='LaviLa', self_attn=False):

@@ -83,7 +83,7 @@ typedef struct {
   int nhead;             /* C / nhead must be 64 */
   int num_layers;        /* 6 */
   int dim_feedforward;   /* 2048 */
-  int num_queries;       /* Q = nq + 1 <= 16 */
+  int num_queries;       /* Q = nq + 1 <= 32 */
   int num_classes1;      /* num_classes + 1 = 22048 */
   int feature_dim;       /* F: 1024 (L/14) or 768 (B/16) */
   int num_frames;        /* T the position embedding was built for */
@@ -247,12 +247,13 @@ int hh_f32_to_bf16(const float* src, void* dst, int64_t n, void* stream);
 /* Divided attention on packed qkv bf16 [B*(1+T*n), 3*H*64] with q pre-scaled -> out bf16 [B*(1+T*n), H*64].
  * kind 0 = space, 1 = time (patch rows), 2 = CLS row. */
 int hh_attention(const void* qkv, void* out, int B, int T, int n, int H, int kind, void* stream);
-/* Query->patch cross attention (tfm_decoder.py:438-441 core): q fp32 [B*Q, heads*64] pre-scaled, K/V bf16 [B*S, ldkv]. */
+/* Query->patch cross attention (tfm_decoder.py:438-441 core): q fp32 [B*Q, heads*64] pre-scaled, K/V bf16 [B*S, ldkv].
+ * 1 <= Q <= 32 (-2 otherwise). */
 int hh_cross_attention(const float* q, const void* K, const void* V, int ldkv, float* out, int B, int Q, int heads,
                        int S, void* stream);
 /* Causal self-attention core of the text tower: qkv bf16 [G*L, 3*H*64] (q pre-scaled) -> out bf16 [G*L, H*64]. */
 int hh_attention_causal(const void* qkv, void* out, int G, int L, int H, void* stream);
-/* Same operator on the fp32 SIMT kernel (second implementation kept for differential testing). */
+/* Same operator on the fp32 SIMT kernel (second implementation kept for differential testing): 1 <= Q <= 16 only. */
 int hh_cross_attention_simt(const float* q, const void* K, const void* V, int ldkv, float* out, int B, int Q, int heads,
                             int S, void* stream);
 
@@ -338,11 +339,11 @@ int hh_linear_f32_backward(const float* dY, int ldy, const float* Y, int ldyo, i
 int hh_layernorm_backward(const float* x, int ldx, const float* w, float eps, const float* dy, int lddy, float* dx,
                           float* dgamma, float* dbeta, int M, int D, void* stream);
 /* Backward of the query self-attention core (hh_decoder's self_attn): q,k,v fp32 rows with stride ld (q pre-scaled),
- * dO fp32 [B*Q, heads*64] -> dq, dk, dv rows with stride ldg. */
+ * dO fp32 [B*Q, heads*64] -> dq, dk, dv rows with stride ldg.  1 <= Q <= 32. */
 int hh_self_attention_backward(const float* q, const float* k, const float* v, int ld, const float* dO, float* dq,
                                float* dk, float* dv, int ldg, int B, int Q, int heads, void* stream);
 /* Backward of hh_cross_attention: O = forward output, dO its gradient (fp32 [B*Q, heads*64]) -> dq fp32 [B*Q, heads*64],
- * dK / dV bf16 rows [B*S] with stride lddkv. */
+ * dK / dV bf16 rows [B*S] with stride lddkv.  1 <= Q <= 32. */
 int hh_cross_attention_backward(const float* q, const void* K, const void* V, int ldkv, const float* O, const float* dO,
                                 float* dq, void* dK, void* dV, int lddkv, int B, int Q, int heads, int S, void* stream);
 
